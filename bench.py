@@ -28,6 +28,15 @@ Multi-GPU: column-sharded, no collective.  gauss_c2 scales weakly (every rank sk
 own 2^22 x 512 block); srht_c3 is the fixed 2^24 x 1024 block split by columns (strong);
 rangefinder_c5 is the fixed block split by rows (strong).
 Prints ONE JSON line on rank 0.
+
+    python bench.py --dump-outputs bench_out ...
+
+also writes, on rank 0, the sketch that each workload timed in this file (the primary one and,
+beside gauss_c2, srht_c3, srht_c1 and gauss_c2_f32) computed in its last timed step, as
+bench_out/<workload>.npy (float64, m x k).  A sketch larger than 16 MB is cut to a fixed,
+seeded sample of its rows, so the files stay under 64 MB in all.  The input blocks come from seeded generators, so two
+builds run with the same arguments can be compared file by file.  A workload whose block had
+to be cut to the free memory is not written (its note in the JSON line says so).
 """
 import argparse
 import json
@@ -80,7 +89,23 @@ def parse():
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary SRHT result")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the sketch of the last timed step of every workload as DIR/<workload>.npy")
     return ap.parse_args()
+
+
+DUMP_BYTES_PER_OUTPUT = 16_000_000       # at most four sketches are dumped: 64 MB in all
+
+
+def dump_sample(out):
+    """`out` (m, k) on the device -> host float64 array: all of it, or the rows of a fixed seeded
+    sample (in ascending order) when it is larger than DUMP_BYTES_PER_OUTPUT."""
+    import torch
+    rows = max(1, DUMP_BYTES_PER_OUTPUT // (out.shape[1] * 8))
+    if out.shape[0] > rows:
+        idx = np.sort(np.random.RandomState(0).choice(out.shape[0], rows, replace=False))
+        out = out[torch.from_numpy(idx).to(out.device)]
+    return out.to(torch.float64).cpu().numpy()
 
 
 def measured_peaks():
@@ -293,6 +318,7 @@ def run_ours(args):
         return x
 
     flush_buf = []
+    dumps = {}
 
     def timed(step, steps, warmup, flush=False):
         """K timed steps.  Default: back to back, start-to-end CUDA events.  flush=True (inputs that
@@ -397,6 +423,11 @@ def run_ours(args):
                         algorithmic="m*n*8 (read U once) + m*k*8 (write sketch) + n (signs) + 4k (indices) bytes per launch")
         small = m_loc * n * esz < 2e8                        # fits L2: flush between steps
         ms, launches, clocks = timed(step, steps, warmup, flush=small)
+        if args.dump_outputs and rank == 0:
+            if note:                                         # another block than the seeded one: not comparable
+                sys.stderr.write(f"bench.py: no {name}.npy written ({note})\n")
+            else:
+                dumps[name] = dump_sample(out)
         t_step = ms / steps / 1e3
         achieved = work / t_step / (1e12 if roof["bound"] == "tensor" else 1e9)
         traffic, traffic_src = None, None
@@ -528,6 +559,10 @@ def run_ours(args):
                    "sample": f"{ms_} of {m} vectors, srht() incl. its per-call sign/index draw: {dt:.1f} s; scaled per vector",
                    "host_cpus": os.cpu_count(), "cols_per_s": m / full}
 
+    if dumps:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if rank == 0:
         line = {
             "metric": "sketch throughput", "value": primary["value"], "unit": "GB/s", "n_gpus": world,
@@ -546,6 +581,8 @@ def run_ours(args):
 def main():
     args = parse()
     assert args.warmup >= 0 and args.steps >= 1
+    if args.impl == "reference" and args.dump_outputs:
+        raise SystemExit("bench.py: --dump-outputs writes the sketches of our arm; the reference arm has none to write")
     if args.impl == "reference":
         run_reference(args)
     else:

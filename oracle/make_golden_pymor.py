@@ -17,6 +17,8 @@ import sys
 import numpy as np
 import scipy.sparse as sp
 
+from oracle import golden_archive
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(ROOT, "tests", "golden")
 REFERENCE = "/root/reference"
@@ -146,7 +148,7 @@ def make_embeddings(E):
     meta["vectorized"] = dict(k1=k1, n_vectors=nv, k2=k2, seed=31, apply_adjoint_is_none=vec.apply_adjoint(None) is None,
                               range_dim_option=int(vec.options["range_dim"]))
     out["__meta__"] = np.array(json.dumps(meta))
-    np.savez_compressed(os.path.join(OUT, "embeddings_reference.npz"), **out)
+    golden_archive.save(os.path.join(OUT, "embeddings_reference.npz"), out)   # equal attributes stored once
     return len(out)
 
 

@@ -39,6 +39,12 @@ def emb_golden():
     return np.load(os.path.join(GOLDEN, "embeddings_transcribed.npz"))
 
 
+def emb_reference():
+    """embeddings_reference.npz: equal attributes are stored once (oracle/golden_archive.py)."""
+    from oracle import golden_archive
+    return golden_archive.load(os.path.join(GOLDEN, "embeddings_reference.npz"))
+
+
 def rel_fro(a, b):
     a = np.asarray(a)
     b = np.asarray(b)

@@ -51,6 +51,24 @@ def test_reference_arm_json_line(monkeypatch, capsys):
     assert capsys.readouterr().out == ""
 
 
+def test_dump_outputs_option_and_sample(monkeypatch):
+    import numpy as np
+    import torch
+    bench = _load_bench()
+    monkeypatch.setattr(sys, "argv", ["bench.py"])
+    assert bench.parse().dump_outputs is None
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--dump-outputs", "d", "--steps", "2"])
+    args = bench.parse()
+    assert args.dump_outputs == "d" and args.steps == 2
+    small = torch.randn(512, 2000, dtype=torch.float64)                 # gauss_c2: 8 MB, kept whole
+    assert np.array_equal(bench.dump_sample(small), small.numpy())
+    big = torch.randn(1024, 4000, dtype=torch.float64)                  # srht_c3: 33 MB, a fixed sample of rows
+    a = bench.dump_sample(big)
+    assert a.dtype == np.float64 and a.shape == (500, 4000) and 4 * a.nbytes <= 64e6
+    rows = np.sort(np.random.RandomState(0).choice(1024, 500, replace=False))
+    assert np.array_equal(a, big.numpy()[rows]) and rows[-1] >= 500    # the seeded rows, not the first 500
+
+
 def test_reference_arm_lifts_the_thread_limit_torchrun_sets(monkeypatch):
     """torchrun exports OMP_NUM_THREADS=1; the CPU arm must still use every host core."""
     bench = _load_bench()

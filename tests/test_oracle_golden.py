@@ -170,3 +170,21 @@ def test_factorization_oracle_identities():
     Q = fo.lu_to_cholesky(S)
     assert abs(Q.conj().T @ Q - S).max() < 1e-10
     assert np.linalg.norm(fo.inverse_lu_apply(fo.factorize(S, symetric=True), V) @ S.T - V) / np.linalg.norm(V) < 1e-10
+
+
+def test_golden_archive_stores_equal_arrays_once(tmp_path):
+    from oracle import golden_archive
+    rs = np.random.RandomState(0)
+    m = rs.standard_normal((33, 301))
+    other = m.copy()
+    other[7, 9] = np.nextafter(other[7, 9], np.inf)                 # one ulp apart: stored on its own
+    arrays = {"a__matrix": m, "a__random_matrix": m.copy(), "a__as_range_array": np.ascontiguousarray(m.T),
+              "a__other": other, "a__int": np.arange(5), "a__float": np.arange(5.0), "__meta__": np.array("{}")}
+    path = str(tmp_path / "g.npz")
+    golden_archive.save(path, arrays)
+    assert sorted(np.load(path).files) == sorted(["a__matrix", "a__other", "a__int", "a__float", "__meta__",
+                                                  golden_archive.ALIASES])
+    z = golden_archive.load(path)
+    assert sorted(z.files) == sorted(arrays) and "a__as_range_array" in z and golden_archive.ALIASES not in z
+    for name, a in arrays.items():
+        assert z[name].dtype == a.dtype and z[name].shape == a.shape and z[name].tobytes() == a.tobytes(), name

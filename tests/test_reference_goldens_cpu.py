@@ -12,14 +12,14 @@ import scipy.sparse as sp
 import oracle
 from oracle import embeddings_oracle as eo
 from oracle import reductor_oracle as ro
-from golden_util import GOLDEN, rel_fro
+from golden_util import GOLDEN, emb_reference, rel_fro
 
 TOL = 1e-12
 
 
 @pytest.fixture(scope="module")
 def emb():
-    z = np.load(os.path.join(GOLDEN, "embeddings_reference.npz"))
+    z = emb_reference()
     return z, json.loads(str(z["__meta__"]))
 
 

@@ -10,7 +10,7 @@ import pytest
 import scipy.sparse as sp
 import torch
 
-from golden_util import GOLDEN, rel_fro
+from golden_util import GOLDEN, emb_reference, rel_fro
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-12
@@ -25,7 +25,7 @@ def rb():
 
 @pytest.fixture(scope="module")
 def emb():
-    z = np.load(os.path.join(GOLDEN, "embeddings_reference.npz"))
+    z = emb_reference()
     return z, json.loads(str(z["__meta__"]))
 
 
