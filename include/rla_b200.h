@@ -160,6 +160,12 @@ int rla_gauss_apply_explicit_f64(const double *theta_dev, int64_t k, int64_t n, 
  * same device function -- but another architecture may round the last FP32 bits differently.
  * For a Theta that is identical everywhere use options['rng'] = 'mt19937' (host draw, explicit
  * GEMM) or kind 1. */
+/* Kinds 0 and 2 (FP32 normals) run on the int8 tensor cores (Ozaki slices, normwise error bound in
+ * the header of csrc/gemm_i8.cu; one stream synchronisation per call); kind 1, and blocks with a
+ * non-finite entry or one >= 2^900, on the FP64 tensor pipe.
+ * ws_dev: rla_gemm_rng_workspace_bytes(m, k_blk, n) (about 8 bytes per element of u more than
+ * rla_gemm_workspace_bytes: the int8 slices of u). */
+size_t rla_gemm_rng_workspace_bytes(int64_t m, int64_t k, int64_t n);
 int rla_embed_apply_rng_f64(uint64_t seed, int kind, double scale,
                             int64_t row0, int64_t k_blk, int64_t col0, int64_t n,
                             const double *u_dev, int64_t m, int64_t ldu,

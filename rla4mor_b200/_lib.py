@@ -39,6 +39,7 @@ _SIGS = {
     "rla_srht_adjoint_f64": (c_int, [_vp, c_int64, _vp, _vp, c_int64, _vp, c_int64, c_int64, c_double, _vp, c_int64,
                                      _vp, c_size_t, _vp]),
     "rla_gemm_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
+    "rla_gemm_rng_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "rla_philox4x32_10_host": (c_int, [_vp, c_int64, _vp]),
     "rla_philox4x32_10_device": (c_int, [_vp, c_int64, _vp, _vp]),
     "rla_dmma_peak_tflops": (c_int, [POINTER(c_double), _vp, _vp]),

@@ -632,6 +632,11 @@ static int sketch_gemm(int mode, const double *theta, int64_t ldt, uint64_t seed
     return RLA_OK;
 }
 
+// gemm_i8.cu: kinds 0 and 2 on the int8 tensor cores
+size_t gemm_i8_workspace_bytes(int64_t m, int64_t k, int64_t n);
+int sketch_gemm_i8(int kind, uint64_t seed, int64_t row0, int64_t col0, const double *u, int64_t m, int64_t ldu,
+                   int64_t k, int64_t n, void *ws, size_t ws_bytes, cudaStream_t st, int64_t *nchunks, bool *ran);
+
 }  // namespace rla
 
 using namespace rla;
@@ -695,6 +700,11 @@ extern "C" size_t rla_gemm_workspace_bytes(int64_t m, int64_t k, int64_t n) {
     return (size_t)std::max(p.max_chunks(), q.max_chunks()) * m * k * sizeof(double);
 }
 
+// kinds 0 and 2 try the int8 path first (gemm_i8.cu) and fall back to DMMA in the same workspace
+extern "C" size_t rla_gemm_rng_workspace_bytes(int64_t m, int64_t k, int64_t n) {
+    return std::max(rla_gemm_workspace_bytes(m, k, n), gemm_i8_workspace_bytes(m, k, n));
+}
+
 extern "C" int rla_gauss_apply_explicit_f64(const double *theta, int64_t k, int64_t n, int64_t ldt, const double *u,
                                             int64_t m, int64_t ldu, double *y, int64_t ldy, void *ws,
                                             size_t ws_bytes, void *stream) {
@@ -724,6 +734,23 @@ extern "C" int rla_embed_apply_rng_f64(uint64_t seed, int kind, double scale, in
     if (m == 0 || k_blk == 0) return RLA_OK;
     RLA_REQUIRE(u && y && ws, "rla_embed_apply_rng_f64: null pointer");
     RLA_REQUIRE(tma_ok(u, ldu), "rla_embed_apply_rng_f64: u must be 16-byte aligned with an even leading dimension");
+    if (kind != 1) {
+        // Theta of kinds 0 and 2 is FP32: Ozaki slices on the int8 tensor cores, unless a block holds a
+        // non-finite entry or one near the FP64 overflow limit (then DMMA, FP64 semantics)
+        cudaStream_t st = (cudaStream_t)stream;
+        int64_t nchunks = 0;
+        bool ran = false;
+        const int rc = sketch_gemm_i8(kind, seed, row0, col0, u, m, ldu, k_blk, n, ws, ws_bytes, st, &nchunks, &ran);
+        if (rc != RLA_OK) return rc;
+        if (ran) {
+            const int64_t tot = m * k_blk;
+            gemm_reduce_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(
+                static_cast<double *>(ws), nchunks, 0, k_blk, m, k_blk, scale, y, ldy, accumulate);
+            count_launch();
+            RLA_CUDA_CHECK(cudaGetLastError());
+            return RLA_OK;
+        }
+    }
     return sketch_gemm(kind + 1, nullptr, 0, seed, scale, row0, col0, u, m, ldu, k_blk, n, y, ldy,
                        accumulate, ws, ws_bytes, (cudaStream_t)stream);
 }

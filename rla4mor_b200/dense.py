@@ -81,7 +81,14 @@ def embed_apply_rng(seed, kind, scale, k, u, row0=0, col0=0, out=None, accumulat
     """Sketch u (m, n) with rows [row0, row0 + k) and columns [col0, col0 + n) of the
     virtual matrix scale * g(seed, row, col); the matrix is never materialised.
 
-    float64 blocks run on the FP64 tensor pipe (csrc/gemm.cu).  float32 blocks with a Theta that
+    float64 blocks with the FP32 normals of KIND_NORMAL / KIND_NORMAL_TF32 run on the int8 tensor
+    cores (csrc/gemm_i8.cu: Theta and per-2^14-column-block scaled U cut into eight 7-bit slices,
+    36 exact int8 slice products, FP64 accumulation).  Its error is bounded NORMWISE, about
+    2^-49 sqrt(2^14) ||u|| ||theta|| per entry whatever the dynamic range of u (the exact bound is in
+    the header of gemm_i8.cu); the componentwise bound in sum |theta| |u| of an FP64 dot product is
+    not kept: an entry far below the largest of its 2^14-column block loses its low bits.  Blocks
+    with a non-finite entry or one near the FP64 overflow limit, and KIND_RADEMACHER, run on the
+    FP64 tensor pipe (csrc/gemm.cu).  float32 blocks with a Theta that
     is exact in TF32 (KIND_RADEMACHER, KIND_NORMAL_TF32) run on the generation-5 tensor cores
     (csrc/gemm32.cu: tcgen05 kind::tf32, two-part split of the block, FP64 accumulation of the
     64-term partial sums); the sketch comes back as float64 either way."""
@@ -111,7 +118,7 @@ def embed_apply_rng(seed, kind, scale, k, u, row0=0, col0=0, out=None, accumulat
     if m == 0 or k == 0:
         return out
     with torch.cuda.device(u.device):
-        ws = _workspace(lib().rla_gemm_workspace_bytes(m, k, n), u.device)
+        ws = _workspace(lib().rla_gemm_rng_workspace_bytes(m, k, n), u.device)
         check(lib().rla_embed_apply_rng_f64(int(seed) & (2 ** 64 - 1), int(kind), float(scale), int(row0), int(k),
                                             int(col0), n, u.data_ptr(), m, _ld(u), out.data_ptr(), out.stride(0),
                                             1 if accumulate else 0, ws.data_ptr(), ws.numel(), stream_ptr()),
