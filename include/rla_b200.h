@@ -191,6 +191,55 @@ int rla_theta_materialize_f64(uint64_t seed, int kind, double scale,
                               int64_t row0, int64_t rows, int64_t col0, int64_t cols,
                               double *out_dev, int64_t ldo, void *stream);
 
+/* ------------------------------------------- MT19937 Gaussian Theta ---------
+ * The reference draws Theta (and every block of the block embedding) on the host with
+ * np.random.RandomState(seed).normal(size=(k, n), loc=0, scale=1/sqrt(k))   rla/embeddings.py:269,458.
+ * These entry points produce the same numbers on the device, bit for bit, for a FRESH RandomState
+ * (pos = 624, no cached Gaussian).  Output 2p of a stream is scale * f * x2 and output 2p + 1 is
+ * scale * f * x1 of its p-th accepted polar attempt (csrc/mt19937.cuh states the arithmetic and the
+ * exactness argument: an extended-precision log, with the pairs whose log lies within w ulp of a
+ * rounding midpoint finished with the C library's log on the host; w = 1/32 by default, 0.5 sends
+ * every pair through the host).
+ *
+ * Plan (host object + caller-owned device workspace), once per batch of streams:
+ *   keys: nstreams x 624 words, RandomState(seed).get_state(legacy=False)['state']['key'];
+ *   nseg[i]: segments of rla_mt19937_segment_words() words given to stream i (enough for its
+ *   normals: 2 * rla_mt19937_plan_pairs(plan, i) normals are available after the build; the caller
+ *   re-plans with more segments if that falls short).
+ *   rla_mt19937_plan_build jumps to every segment start (F2 jump-ahead), counts the accepted
+ *   attempts of every segment and scans them; it synchronises the stream once.  The workspace must
+ *   stay allocated and untouched while the plan is used.
+ * Execute: normals [first[i], first[i] + count[i]) of stream i go to out_dev + offset[i]
+ *   (out_len elements in all); first may be odd.  ws_dev: rla_mt19937_execute_workspace_bytes(plan,
+ *   flag_cap), room for flag_cap flagged pairs; staging_host: flag_cap doubles of pinned host memory
+ *   (NULL only if nothing can be flagged).  *nflagged receives the number of flagged pairs; when it
+ *   exceeds flag_cap the call returns RLA_ERR_WORKSPACE and the caller retries with a larger one.
+ *   Synchronises the stream once after the write pass and, when pairs were flagged, twice more
+ *   around the host fix-up (their r2 down, libm's log up). */
+typedef struct rla_mt19937_plan rla_mt19937_plan;
+int64_t rla_mt19937_segment_words(void);
+int rla_mt19937_plan_create(rla_mt19937_plan **plan, const uint32_t *keys, const int64_t *nseg, int64_t nstreams);
+void rla_mt19937_plan_destroy(rla_mt19937_plan *plan);
+size_t rla_mt19937_plan_workspace_bytes(const rla_mt19937_plan *plan);
+int rla_mt19937_plan_build(rla_mt19937_plan *plan, void *ws_dev, size_t ws_bytes, void *stream);
+/* accepted pairs available to stream i after the build (-1 before it) */
+int64_t rla_mt19937_plan_pairs(const rla_mt19937_plan *plan, int64_t i);
+size_t rla_mt19937_execute_workspace_bytes(const rla_mt19937_plan *plan, int64_t flag_cap);
+int rla_mt19937_normal_f64(const rla_mt19937_plan *plan, const int64_t *first, const int64_t *count,
+                           const int64_t *offset, double scale, double w, double *out_dev, int64_t out_len,
+                           void *ws_dev, size_t ws_bytes, int64_t flag_cap, double *staging_host,
+                           int64_t *nflagged, void *stream);
+/* Host-only hooks of the same code (tests):
+ *   rla_mt19937_jump_host: the state `steps` words ahead of key_in (both 624 words, pos = 624);
+ *   rla_mt19937_attempts_host: n attempts from 4n output words (tempered, as random_raw gives them)
+ *   -> x1, x2, r2, accepted;
+ *   rla_mt19937_ext_log_host: the extended log of x in (0, 1) as hi + lo and its midpoint flag;
+ *   rla_libm_log_host: the C library's log of n values (several threads, no vector math library). */
+int rla_mt19937_jump_host(const uint32_t *key_in, uint64_t steps, uint32_t *key_out);
+int rla_mt19937_attempts_host(const uint32_t *words, int64_t n, double *x1, double *x2, double *r2, int8_t *accept);
+int rla_mt19937_ext_log_host(const double *x, int64_t n, double w, double *hi, double *lo, int8_t *flag);
+int rla_libm_log_host(const double *x, int64_t n, double *out);
+
 /* out(m, n) = V(m, k) * Theta(k, n): the adjoint / explicit-matrix product
  * (SrhtEmbedding.apply_adjoint rla/embeddings.py:175-178, rb.lincomb(T.T)
  * mor/sketched_reductor.py:99-100).  Theta is transposed into scratch and the product

@@ -17,6 +17,8 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--shared", "-Xptxas", "-v",
     "-Wno-deprecated-gpu-targets",
 ]
+# NumPy's Gaussian stream is reproduced bit for bit only without contracted multiply-adds
+FILE_FLAGS = {"mt19937.cu": ["--fmad=false", "-Xcompiler", "-ffp-contract=off"]}
 
 
 def _nvcc():
@@ -58,7 +60,8 @@ def build_library(force=False, verbose=False):
                         for h in glob.glob(os.path.join(CSRC, "*.cuh")) +
                         [os.path.join(os.path.dirname(HERE), "include", "rla_b200.h")])):
             continue
-        cmd = [_nvcc()] + [f for f in NVCC_FLAGS if f != "--shared"] + ["-c", src, "-o", obj]
+        cmd = [_nvcc()] + [f for f in NVCC_FLAGS if f != "--shared"] + FILE_FLAGS.get(os.path.basename(src), []) + \
+            ["-c", src, "-o", obj]
         if ccbin:
             cmd += ["-ccbin", ccbin]
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, env=env)))

@@ -51,6 +51,19 @@ _SIGS = {
     "rla_embed_apply_rng_f32": (c_int, [c_uint64, c_int, c_double, c_int64, c_int64, c_int64, c_int64, _vp, c_int64,
                                         c_int64, _vp, c_int64, c_int, _vp, c_size_t, _vp]),
     "rla_theta_materialize_f64": (c_int, [c_uint64, c_int, c_double, c_int64, c_int64, c_int64, c_int64, _vp, c_int64, _vp]),
+    "rla_mt19937_segment_words": (c_int64, []),
+    "rla_mt19937_plan_create": (c_int, [POINTER(c_void_p), _vp, _vp, c_int64]),
+    "rla_mt19937_plan_destroy": (None, [_vp]),
+    "rla_mt19937_plan_workspace_bytes": (c_size_t, [_vp]),
+    "rla_mt19937_plan_build": (c_int, [_vp, _vp, c_size_t, _vp]),
+    "rla_mt19937_plan_pairs": (c_int64, [_vp, c_int64]),
+    "rla_mt19937_execute_workspace_bytes": (c_size_t, [_vp, c_int64]),
+    "rla_mt19937_normal_f64": (c_int, [_vp, _vp, _vp, _vp, c_double, c_double, _vp, c_int64, _vp, c_size_t, c_int64,
+                                       _vp, POINTER(c_int64), _vp]),
+    "rla_mt19937_jump_host": (c_int, [_vp, c_uint64, _vp]),
+    "rla_mt19937_attempts_host": (c_int, [_vp, c_int64, _vp, _vp, _vp, _vp]),
+    "rla_mt19937_ext_log_host": (c_int, [_vp, c_int64, c_double, _vp, _vp, _vp]),
+    "rla_libm_log_host": (c_int, [_vp, c_int64, _vp]),
     "rla_gemm_nn_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "rla_gemm_nn_f64": (c_int, [_vp, c_int64, c_int64, c_int64, _vp, c_int64, c_int64, _vp, c_int64, _vp, c_size_t, _vp]),
     "rla_spmm_csr_f64": (c_int, [_vp, _vp, _vp, c_int64, c_int64, _vp, c_int64, c_int64, _vp, c_int64, _vp]),

@@ -15,10 +15,12 @@ for pyMOR VectorArrays, see vectorarray.py), or plain NumPy arrays / CUDA tensor
 in which case the result comes back as the same kind.
 
 One option is new: `options['rng']`
-  * 'mt19937' (default): Theta / block seeds are drawn on the host by NumPy's legacy
-    RandomState exactly as the reference does (embeddings.py:269,403,458), uploaded,
-    and applied by the explicit-Theta tensor-core GEMM -- same seed, same Theta, same
-    sketch as the reference to 1e-12;
+  * 'mt19937' (default): Theta is NumPy's legacy RandomState(seed).normal draw, exactly
+    as the reference makes it (embeddings.py:269,458), and is applied by the explicit-Theta
+    tensor-core GEMM -- same seed, same Theta, same sketch as the reference to 1e-12.
+    With a CUDA device the draw itself runs on the GPU (csrc/mt19937.cu: MT19937 jump-ahead,
+    bit-identical to NumPy's stream) and host copies such as `_random_matrix` are downloads
+    of it; without one NumPy draws it.  Block seeds (:403) stay host draws;
   * 'philox' / 'philox_rademacher': Theta is generated on the fly inside the GEMM
     from a counter-based RNG and never materialised (the only way k x n = 2000 x 2**22
     fits anywhere); `get_random_matrix()` exports exactly what the kernel used;
@@ -37,6 +39,7 @@ from . import dense
 from .srht import SrhtPlan, draw_signs_and_indices
 from ._lib import check, lib, require_cuda, stream_ptr
 from .vectorarray import DeviceVectorArray, DeviceVectorSpace, IdentityOperator, as_device_block
+from . import mt19937
 
 _logger = logging.getLogger("rla4mor_b200.embeddings")
 _warned_once = set()
@@ -78,6 +81,14 @@ class Concatenation:
     def __matmul__(self, other):
         ops = other.operators if isinstance(other, Concatenation) else (other,)
         return Concatenation(self.operators + tuple(ops))
+
+
+def _cuda_available():
+    try:
+        import torch
+    except ImportError:
+        return False
+    return torch.cuda.is_available()
 
 
 def _wrap_result(kind, space, t):
@@ -505,7 +516,11 @@ class GaussianEmbedding(RandomEmbedding):
         n = self.sqrt_product.range.dim
         seed = self._seed
         if self._rng_mode == "mt19937":
-            return np.random.RandomState(seed).normal(size=(k, n), loc=0, scale=1 / np.sqrt(k))
+            if not _cuda_available():
+                return np.random.RandomState(seed).normal(size=(k, n), loc=0, scale=1 / np.sqrt(k))
+            # the device draw is kept: apply() and get_matrix_device() use it without an upload
+            self._theta_dev = mt19937.gaussian_matrix([seed], [k], n, 1 / np.sqrt(k))
+            return self._theta_dev.cpu().numpy()
         return dense.theta_materialize(seed, self._kind(), 1.0 / np.sqrt(k), k, n).cpu().numpy()
 
     def _compute_random_matrix_device(self):
@@ -513,11 +528,9 @@ class GaussianEmbedding(RandomEmbedding):
         k = self.range.dim
         n = self.sqrt_product.range.dim
         if self._rng_mode == "mt19937":
-            # the reference's Theta is a host MT19937 draw (that is what makes it bit-identical);
-            # it is uploaded once and shared with apply()
+            # NumPy's MT19937 draw made on the device; shared with apply()
             if self._theta_dev is None:
-                gauss = self._random_matrix if self._random_matrix is not None else self._compute_random_matrix()
-                self._theta_dev = torch.from_numpy(gauss).cuda()
+                self._theta_dev = mt19937.gaussian_matrix([self._seed], [k], n, 1 / np.sqrt(k))
             return self._theta_dev
         return dense.theta_materialize(self._seed, self._kind(), 1.0 / np.sqrt(k), k, n)
 
@@ -671,20 +684,39 @@ class BlockGaussianEmbedding(RandomEmbedding):
             V = V.to(torch.float64)
         k = self.range.dim
         result = torch.empty((V.shape[0], k), dtype=torch.float64, device=V.device)
+        # one plan (jump-ahead + acceptance count) for the streams of all blocks
+        plan = self._block_plan(V.device) if self._rng_mode == "mt19937" else None
         off = 0
         for i in range(len(self.block_sizes)):
             b = self.block_sizes[i]
-            result[:, off:off + b].copy_(self._apply_block(i, V))
+            result[:, off:off + b].copy_(self._apply_block(i, V, plan))
             off += b
         return _wrap_result(kind, self.range, result)
 
-    def _apply_block(self, i, V):
-        """(m, b_i) sketch of the CUDA block V (already Q U) by row block i of Theta (:430-432)."""
+    def _block_plan(self, device):
+        n = self.sqrt_product.range.dim
+        return mt19937.NormalPlan(list(self.block_seeds), [b * n for b in self.block_sizes], device)
+
+    def _draw_block_device(self, i, plan):
+        """Row block i of Theta drawn on the device from a plan over all blocks."""
         import torch
+        k = self.range.dim
+        n = self.sqrt_product.range.dim
+        b = self.block_sizes[i]
+        out = torch.empty((b, n), dtype=torch.float64, device=plan.device)
+        count = np.zeros(self.n_blocks, np.int64)
+        count[i] = b * n
+        if out.numel():
+            plan.execute(out.view(-1), 0, count, 0, 1 / np.sqrt(k))
+        return out
+
+    def _apply_block(self, i, V, plan=None):
+        """(m, b_i) sketch of the CUDA block V (already Q U) by row block i of Theta (:430-432)."""
         k = self.range.dim
         b = self.block_sizes[i]
         if self._rng_mode == "mt19937":
-            gauss = torch.from_numpy(self._get_random_block(i)).to(V.device)
+            # Theta blocks are not kept (the reference draws them again on every apply)
+            gauss = self._draw_block_device(i, plan if plan is not None else self._block_plan(V.device))
             return dense.gauss_apply_explicit(gauss, V)
         # independent stream per block: the block's own seed, rows 0..b-1
         return dense.embed_apply_rng(int(self.block_seeds[i]), self._kind(), 1.0 / np.sqrt(k), b, V)
@@ -693,6 +725,10 @@ class BlockGaussianEmbedding(RandomEmbedding):
         return self._adjoint_sqrt_product(self._compute_random_matrix())
 
     def _compute_random_matrix(self):                                      # :444-450
+        if self._rng_mode == "mt19937" and _cuda_available():
+            k = self.range.dim
+            return mt19937.gaussian_matrix_host(list(self.block_seeds), self.block_sizes, self.sqrt_product.range.dim,
+                                                1 / np.sqrt(k))
         return np.vstack([self._get_random_block(i) for i in range(self.n_blocks)])
 
     def _get_random_block(self, ind):                                      # :452-461
@@ -701,18 +737,20 @@ class BlockGaussianEmbedding(RandomEmbedding):
         b = self.block_sizes[ind]
         seed = self.block_seeds[ind]
         if self._rng_mode == "mt19937":
-            return np.random.RandomState(seed).normal(size=(b, n), loc=0, scale=1 / np.sqrt(k))
+            if not _cuda_available():
+                return np.random.RandomState(seed).normal(size=(b, n), loc=0, scale=1 / np.sqrt(k))
+            return mt19937.gaussian_matrix([seed], [b], n, 1 / np.sqrt(k)).cpu().numpy()
         return dense.theta_materialize(int(seed), self._kind(), 1.0 / np.sqrt(k), b, n).cpu().numpy()
 
     def get_block(self, ind):                                              # :463-467
         return self._adjoint_sqrt_product(self._get_random_block(ind))
 
     def _get_random_block_device(self, ind):
-        torch = require_cuda()
-        if self._rng_mode == "mt19937":
-            return torch.from_numpy(self._get_random_block(ind)).cuda()
+        require_cuda()
         k = self.range.dim
         n = self.sqrt_product.range.dim
+        if self._rng_mode == "mt19937":
+            return mt19937.gaussian_matrix([self.block_seeds[ind]], [self.block_sizes[ind]], n, 1 / np.sqrt(k))
         return dense.theta_materialize(int(self.block_seeds[ind]), self._kind(), 1.0 / np.sqrt(k), self.block_sizes[ind], n)
 
     def get_block_device(self, ind):
@@ -721,4 +759,8 @@ class BlockGaussianEmbedding(RandomEmbedding):
 
     def _compute_random_matrix_device(self):
         import torch
+        if self._rng_mode == "mt19937":
+            require_cuda()
+            return mt19937.gaussian_matrix(list(self.block_seeds), self.block_sizes, self.sqrt_product.range.dim,
+                                           1 / np.sqrt(self.range.dim))
         return torch.cat([self._get_random_block_device(i) for i in range(self.n_blocks)], dim=0)
