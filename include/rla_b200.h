@@ -190,6 +190,23 @@ int rla_embed_apply_rng_f32(uint64_t seed, int kind, double scale,
 int rla_theta_materialize_f64(uint64_t seed, int kind, double scale,
                               int64_t row0, int64_t rows, int64_t col0, int64_t cols,
                               double *out_dev, int64_t ldo, void *stream);
+/* The adjoint of the on-the-fly Gaussian embeddings, Theta generated in the kernel and never
+ * materialised: out(m, n) = V(m, k) * Theta(k, n), all row-major.  Replaces pyMOR's adjoint of the
+ * explicit matrix, V @ get_matrix(), of GaussianEmbedding and BlockGaussianEmbedding
+ * (rla/embeddings.py:214-270, 373-467; Q^H is applied by the caller).
+ * Theta is a stack of nblocks blocks: row_start_dev (nblocks + 1 entries, 0 = row_start[0] <= ... <=
+ * row_start[nblocks] = k) and seeds_dev (nblocks entries) are caller-owned device memory.  Rows
+ * [row_start[b], row_start[b+1]) of Theta are rows 0 .. size_b - 1 of the virtual matrix
+ * scale * g(seeds[b], row, col) of rla_theta_materialize_f64 (kind 0, 1 or 2), each entry formed as
+ * fl(scale * g).  The table is read on the device, so ldv >= k is the caller's to ensure.
+ * Every element of `out` is one DMMA chain over k in ascending order, four terms at a time: the result
+ * equals rla_gemm_nn_f64(V, Theta materialised) bit for bit when that call takes its tensor-pipe path
+ * (16-byte aligned operands, even leading dimensions), and is deterministic from run to run.
+ * One launch, no workspace. */
+int rla_embed_adjoint_rng_f64(int kind, double scale,
+                              const uint64_t *seeds_dev, const int64_t *row_start_dev, int64_t nblocks,
+                              int64_t n, const double *v_dev, int64_t m, int64_t ldv,
+                              double *out_dev, int64_t ldo, void *stream);
 
 /* ------------------------------------------- MT19937 Gaussian Theta ---------
  * The reference draws Theta (and every block of the block embedding) on the host with

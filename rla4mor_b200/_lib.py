@@ -51,6 +51,8 @@ _SIGS = {
     "rla_embed_apply_rng_f32": (c_int, [c_uint64, c_int, c_double, c_int64, c_int64, c_int64, c_int64, _vp, c_int64,
                                         c_int64, _vp, c_int64, c_int, _vp, c_size_t, _vp]),
     "rla_theta_materialize_f64": (c_int, [c_uint64, c_int, c_double, c_int64, c_int64, c_int64, c_int64, _vp, c_int64, _vp]),
+    "rla_embed_adjoint_rng_f64": (c_int, [c_int, c_double, _vp, _vp, c_int64, c_int64, _vp, c_int64, c_int64, _vp,
+                                          c_int64, _vp]),
     "rla_mt19937_segment_words": (c_int64, []),
     "rla_mt19937_plan_create": (c_int, [POINTER(c_void_p), _vp, _vp, c_int64]),
     "rla_mt19937_plan_destroy": (None, [_vp]),

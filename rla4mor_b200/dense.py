@@ -2,10 +2,12 @@
 
 Y(m, k) = U(m, n) Theta(k, n)^T in FP64 on the tensor pipe, with Theta explicit
 (`gauss_apply_explicit`, the reference's `(Theta @ (QU)^T)^T`, rla/embeddings.py:250-254)
-or generated on the fly from the counter-based RNG (`embed_apply_rng`), plus the export
-of what that generator produces (`theta_materialize`, parity tooling).
+or generated on the fly from the counter-based RNG (`embed_apply_rng`), the adjoint
+V(m, k) Theta(k, n) with the same on-the-fly Theta (`embed_adjoint_rng`, csrc/adjoint_rng.cu),
+plus the export of what that generator produces (`theta_materialize`, parity tooling).
 All inputs are CUDA tensors; there is no CPU path.
 """
+import numpy as np
 import torch
 
 from ._lib import check, lib, stream_ptr
@@ -123,6 +125,35 @@ def embed_apply_rng(seed, kind, scale, k, u, row0=0, col0=0, out=None, accumulat
                                             int(col0), n, u.data_ptr(), m, _ld(u), out.data_ptr(), out.stride(0),
                                             1 if accumulate else 0, ws.data_ptr(), ws.numel(), stream_ptr()),
               "rla_embed_apply_rng_f64")
+    return out
+
+
+def embed_adjoint_rng(seeds, row_starts, kind, scale, v, n):
+    """out(m, n) = v(m, k) @ Theta(k, n) with Theta generated in the kernel (csrc/adjoint_rng.cu),
+    never materialised.  Theta stacks len(seeds) blocks: rows [row_starts[b], row_starts[b + 1]) are
+    rows 0 .. size_b - 1 of the virtual matrix scale * g(seeds[b], row, col) that `theta_materialize`
+    exports.  Bit-identical to `gemm_nn(v, Theta)` when that product runs on its tensor-pipe path
+    (16-byte aligned operands, even leading dimensions).  A float32 v is widened to float64."""
+    seeds = np.asarray([int(s) & (2 ** 64 - 1) for s in seeds], dtype=np.uint64)
+    row_starts = np.asarray(row_starts, dtype=np.int64)
+    nblocks = len(seeds)
+    assert nblocks >= 1 and row_starts.shape == (nblocks + 1,) and row_starts[0] == 0, "bad block table"
+    assert np.all(np.diff(row_starts) >= 0) and np.all(np.diff(row_starts) < 2 ** 32), "bad block table"
+    if v.dtype == torch.float32:
+        v = v.to(torch.float64)
+    v = _rows(v)
+    assert v.dtype == torch.float64
+    m, k = v.shape
+    n = int(n)
+    assert k == row_starts[-1], f"v has {k} columns, the blocks {row_starts[-1]} rows"
+    out = torch.empty((m, n), dtype=torch.float64, device=v.device)
+    if m == 0 or n == 0:
+        return out
+    with torch.cuda.device(v.device):
+        table = torch.from_numpy(np.concatenate([seeds.view(np.int64), row_starts])).to(v.device)
+        check(lib().rla_embed_adjoint_rng_f64(int(kind), float(scale), table.data_ptr(), table[nblocks:].data_ptr(),
+                                              nblocks, n, v.data_ptr(), m, _ld(v), out.data_ptr(), out.stride(0),
+                                              stream_ptr()), "rla_embed_adjoint_rng_f64")
     return out
 
 

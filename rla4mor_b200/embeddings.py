@@ -23,7 +23,8 @@ One option is new: `options['rng']`
     of it; without one NumPy draws it.  Block seeds (:403) stay host draws;
   * 'philox' / 'philox_rademacher': Theta is generated on the fly inside the GEMM
     from a counter-based RNG and never materialised (the only way k x n = 2000 x 2**22
-    fits anywhere); `get_random_matrix()` exports exactly what the kernel used;
+    fits anywhere), by `apply` and by `apply_adjoint` alike (csrc/adjoint_rng.cu generates it
+    inside the adjoint's product); `get_random_matrix()` exports exactly what the kernels used;
   * 'philox_tf32': the normals of 'philox' rounded to TF32 (10 explicit mantissa bits).
     With this mode (and with 'philox_rademacher') Theta is exact in TF32, and FLOAT32
     blocks are sketched on the generation-5 tensor cores (tcgen05 kind::tf32 with a
@@ -254,6 +255,28 @@ class RandomEmbedding:
         if isinstance(Q, IdentityOperator):
             return rmat
         return Q.apply_adjoint(Q.range.from_numpy(rmat.conj())).to_numpy().conj()
+
+    def _gaussian_adjoint(self, U, product, includes_sqrt_product=False):
+        """V @ get_matrix() of the Gaussian embeddings from `product(v)`, a real CUDA block times
+        the (k, n) matrix: Theta, then Q^H applied here, or the explicit matrix that already holds it
+        (`includes_sqrt_product`).  Theta is real, so a complex block goes through as its real and
+        imaginary parts; that needs an identity sqrt_product, as SrhtEmbedding.apply_adjoint does."""
+        torch = require_cuda()
+        if isinstance(U, DeviceVectorArray):
+            assert U in self.range
+        v, kind = _unwrap(U)
+        assert v.shape[1] == self.range.dim
+        Q = self.sqrt_product
+        if v.is_complex():
+            if not isinstance(Q, IdentityOperator):
+                raise TypeError(f"{type(self).__name__}.apply_adjoint: complex blocks need an identity sqrt_product")
+            m = v.shape[0]
+            w2 = product(torch.cat([v.real, v.imag], dim=0).to(torch.float64))
+            return _wrap_result(kind, self.source, torch.complex(w2[:m], w2[m:]))
+        w = product(v.to(torch.float64))
+        if not includes_sqrt_product and not isinstance(Q, IdentityOperator):
+            w = Q.apply_adjoint(DeviceVectorArray(Q.range, w)).data
+        return _wrap_result(kind, self.source, w)
 
     @property
     def _rng_mode(self):
@@ -499,13 +522,16 @@ class GaussianEmbedding(RandomEmbedding):
         return _wrap_result(kind, self.range, y)
 
     def apply_adjoint(self, U, mu=None):
-        """V @ get_matrix()  (pyMOR's generic adjoint of a matrix operator)."""
-        from .reductor_ops import gemm_nn
-        torch = require_cuda()
-        if isinstance(U, DeviceVectorArray):
-            assert U in self.range
-        v, kind = _unwrap(U)
-        return _wrap_result(kind, self.source, gemm_nn(v.to(torch.float64), self.get_matrix_device()))
+        """V @ get_matrix()  (pyMOR's generic adjoint of a matrix operator).  'mt19937', or a matrix
+        already on the device: the product with that matrix.  Otherwise V Theta with Theta generated
+        in the kernel (csrc/adjoint_rng.cu), then Q^H: Theta is neither materialised nor kept."""
+        if self._rng_mode == "mt19937" or self._matrix_dev is not None:
+            from .reductor_ops import gemm_nn
+            return self._gaussian_adjoint(U, lambda v: gemm_nn(v, self.get_matrix_device()), includes_sqrt_product=True)
+        k = self.range.dim
+        n = self.sqrt_product.range.dim
+        return self._gaussian_adjoint(
+            U, lambda v: dense.embed_adjoint_rng([self._seed], [0, k], self._kind(), 1.0 / np.sqrt(k), v, n))
 
     def _compute_matrix(self):                                             # :258-262
         gauss = self._random_matrix if self._random_matrix is not None else self._compute_random_matrix()
@@ -692,6 +718,31 @@ class BlockGaussianEmbedding(RandomEmbedding):
             result[:, off:off + b].copy_(self._apply_block(i, V, plan))
             off += b
         return _wrap_result(kind, self.range, result)
+
+    def apply_adjoint(self, U, mu=None):
+        """V @ get_matrix()  (pyMOR's adjoint of the explicit matrix, embeddings.py:437-441), then Q^H.
+        On-the-fly modes: one kernel launch over all blocks with Theta generated in the kernel
+        (csrc/adjoint_rng.cu).  'mt19937': one plan for all blocks, each block drawn on the device in
+        turn and V[:, block] @ Theta_b accumulated, so one block of Theta is held at a time."""
+        k = self.range.dim
+        n = self.sqrt_product.range.dim
+        if self._rng_mode != "mt19937":
+            starts = np.concatenate([[0], np.cumsum(self.block_sizes)])
+            return self._gaussian_adjoint(
+                U, lambda v: dense.embed_adjoint_rng([int(s) for s in self.block_seeds], starts, self._kind(),
+                                                     1.0 / np.sqrt(k), v, n))
+
+        def product(v):
+            import torch
+            from .reductor_ops import gemm_nn
+            plan = self._block_plan(v.device)
+            out = torch.zeros((v.shape[0], n), dtype=torch.float64, device=v.device)
+            off = 0
+            for i, b in enumerate(self.block_sizes):
+                out += gemm_nn(v[:, off:off + b], self._draw_block_device(i, plan))
+                off += b
+            return out
+        return self._gaussian_adjoint(U, product)
 
     def _block_plan(self, device):
         n = self.sqrt_product.range.dim
