@@ -349,6 +349,40 @@ int rla_residual_norm_f64(const double *S_dev, int64_t Q, int64_t k, int64_t r,
                           const double *b_dev, int64_t P, const double *tr_dev,
                           double *out_dev, void *stream);
 
+/* ------------------------------------------- ROM over a parameter set ------
+ * The online half of the sketched ROM for P parameter values mu_p at once (csrc/rom_batch.cu).
+ * The affine coefficients are row-major device arrays th_dev (P, Q; row stride ldth) and tf_dev
+ * (P, Pf; row stride ldtf); the ROM's data are in its existing layouts.
+ *
+ * rla_rom_solve_batch_f64 replaces, per mu_p, StationaryModel.solve of the Galerkin ROM
+ * (mor/sketched_reductor.py:165-166; SketchedRom.solve): lhs_dev is Q contiguous row-major r x r
+ * matrices, rhs_dev Pf contiguous r-vectors.  A_p = sum_q th[p, q] A_q and b_p = sum_j tf[p, j] f_j
+ * are assembled in shared memory (ascending q / j, fma), factored by LU with partial pivoting
+ * (largest |.|, ties to the smallest row: LAPACK's rule) and solved; row p of a_dev (row stride lda)
+ * receives a_p.  info_dev[p] (int32) = 0, or i > 0 when U(i, i) is exactly zero (LAPACK's
+ * convention); the row a_p is then NaN.  1 <= r <= rla_rom_solve_batch_max_r() (169: the augmented
+ * r x (r + 1) system fits in the shared memory of one CTA).  One launch, no workspace.
+ *
+ * rla_residual_norm_batch_f64 replaces, per mu_p, ResidualErrorEstimator.estimate_error
+ * (mor/sketched_reductor.py:216-219; the single-mu rla_residual_norm_f64):
+ *   est[p] = || sum_q th[p, q] S_q a_p - sum_j tf[p, j] g_j ||_2
+ * W_dev (N x kp, row stride ldw, N = Q r + Pf) is the stack [S_0^T; ...; S_{Q-1}^T; g_0^T; ...]
+ * of the ROM's (r, kp) row blocks and kp-vectors; a_dev (P, r; row stride lda) holds the reduced
+ * solutions.  The product X(P, N) W with X[p, q r + i] = th[p, q] a[p, i], X[p, Q r + j] = -tf[p, j]
+ * runs on the FP64 tensor pipe with X formed in the kernel; neither X nor the residuals are stored.
+ * ws_dev (caller-owned, rla_residual_norm_batch_workspace_bytes(P, kp) = 8 P ceil(kp / 128) bytes)
+ * receives the per-tile partial sums, added in tile order: bit-identical from run to run.  A NaN
+ * row of a_dev gives a NaN estimate.  Two launches. */
+int rla_rom_solve_batch_max_r(void);
+int rla_rom_solve_batch_f64(const double *lhs_dev, int64_t Q, int64_t r, const double *rhs_dev, int64_t Pf,
+                            const double *th_dev, int64_t ldth, const double *tf_dev, int64_t ldtf, int64_t P,
+                            double *a_dev, int64_t lda, int32_t *info_dev, void *stream);
+size_t rla_residual_norm_batch_workspace_bytes(int64_t P, int64_t kp);
+int rla_residual_norm_batch_f64(const double *W_dev, int64_t ldw, int64_t Q, int64_t r, int64_t Pf, int64_t kp,
+                                const double *th_dev, int64_t ldth, const double *tf_dev, int64_t ldtf,
+                                const double *a_dev, int64_t lda, int64_t P, double *est_dev,
+                                void *ws_dev, size_t ws_bytes, void *stream);
+
 /* --------------------------------------- sparse triangular solves (8f.1) ----
  * Device side of InverseLuOperator.apply / apply_adjoint (utilities/factorization.py:118-132,
  * `slu.solve(V.T).T`): the inverse_product R^-1 in front of the sketch

@@ -73,6 +73,12 @@ _SIGS = {
     "rla_svd_jacobi_f64": (c_int, [_vp, c_int64, c_int64, c_int64, _vp, _vp, _vp, _vp, c_int, c_double,
                                    POINTER(c_int), _vp]),
     "rla_residual_norm_f64": (c_int, [_vp, c_int64, c_int64, c_int64, _vp, _vp, _vp, c_int64, _vp, _vp, _vp]),
+    "rla_rom_solve_batch_max_r": (c_int, []),
+    "rla_rom_solve_batch_f64": (c_int, [_vp, c_int64, c_int64, _vp, c_int64, _vp, c_int64, _vp, c_int64, c_int64,
+                                        _vp, c_int64, _vp, _vp]),
+    "rla_residual_norm_batch_workspace_bytes": (c_size_t, [c_int64, c_int64]),
+    "rla_residual_norm_batch_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, c_int64, _vp, c_int64, _vp,
+                                            c_int64, _vp, c_int64, c_int64, _vp, _vp, c_size_t, _vp]),
     "rla_gram_schmidt_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "rla_gram_schmidt_status_offset": (c_int64, [c_int64, c_int64]),
     "rla_gram_schmidt_ws_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, _vp, _vp, c_double, c_double, c_double,

@@ -309,18 +309,22 @@ def to_affine_model(fom):
 
 
 class ResidualErrorEstimator(ImmutableObject):
-    """mor/sketched_reductor.py:210-219 on the device ROM: the norm is one kernel."""
+    """mor/sketched_reductor.py:210-219 on the device ROM: the norms of all rows of U are one
+    batched estimate (SketchedRom.estimate_error_batch) with theta(mu) repeated."""
 
     def __init__(self, rom_dev, name=None):
         self.__auto_init(locals())
 
     def estimate_error(self, U, mu, m=None):
-        a = U.to_numpy()
-        return np.array([self.rom_dev.estimate_error(a=self._dev_vec(row), mu=mu) for row in a])
-
-    def _dev_vec(self, row):
         import torch
-        return torch.as_tensor(np.ascontiguousarray(row), dtype=torch.float64, device="cuda")
+        a = U.to_numpy()
+        th, tf = self.rom_dev.fom.thetas(mu)
+        rows = len(a)
+        est = self.rom_dev.estimate_error_batch(
+            a=torch.as_tensor(np.ascontiguousarray(a), dtype=torch.float64, device="cuda"),
+            theta_lhs=np.tile(np.asarray(th, dtype=np.float64), (rows, 1)).reshape(rows, len(th)),
+            theta_rhs=np.tile(np.asarray(tf, dtype=np.float64), (rows, 1)).reshape(rows, len(tf)))
+        return est.cpu().numpy()
 
 
 class SketchedReductor(BasicObject):

@@ -6,7 +6,7 @@ import ctypes
 import numpy as np
 import torch
 
-from . import dense
+from . import _lib, dense
 from ._lib import RlaError, check, lib, stream_ptr
 
 
@@ -218,3 +218,115 @@ def residual_norm(S_terms, theta_lhs, b_terms, theta_rhs, a):
         check(lib().rla_residual_norm_f64(S.data_ptr(), Q, k, r, th.data_ptr(), av.data_ptr(), b.data_ptr(), P,
                                           tr.data_ptr(), out.data_ptr(), stream_ptr()), "rla_residual_norm_f64")
     return out
+
+
+# ------------------------------------------------------------- ROM over a parameter set
+def _param_rows(x, P, cols, name, device):
+    """(P, cols) float64 CUDA rows with unit inner stride and its row stride; ValueError on a
+    shape mismatch (raised before anything is copied or launched)."""
+    x = torch.as_tensor(x, dtype=torch.float64)
+    if x.dim() != 2 or tuple(x.shape) != (P, cols):
+        raise ValueError(f"{name}: expected shape ({P}, {cols}), got {tuple(x.shape)}")
+    x = x.to(device)
+    if cols and (x.stride(1) != 1 or (P > 1 and x.stride(0) < cols)):
+        x = x.contiguous()
+    return x, (max(x.stride(0), cols) if P > 1 else cols)
+
+
+def _require_cuda(dev, what):
+    if dev.type != "cuda":
+        raise ValueError(f"{what}: the ROM's data must be CUDA tensors")
+
+
+def _stack(terms, shape, name):
+    """A list of equally shaped tensors (or one stacked tensor) as one contiguous float64 tensor."""
+    if isinstance(terms, torch.Tensor):
+        t = terms
+    else:
+        terms = list(terms)
+        t = torch.stack([torch.as_tensor(x).to(torch.float64) for x in terms]) if terms else torch.empty(shape)
+    if tuple(t.shape) != tuple(shape):
+        raise ValueError(f"{name}: expected shape {tuple(shape)}, got {tuple(t.shape)}")
+    return t
+
+
+def rom_solve_batch_max_r():
+    """Largest reduced dimension r of rom_solve_batch (the r x (r + 1) system in one CTA's shared memory)."""
+    return int(lib().rla_rom_solve_batch_max_r())
+
+
+def rom_solve_batch(lhs, rhs, th, tf, check=True):
+    """Reduced Galerkin solves  (sum_q th[p, q] A_q) a_p = sum_j tf[p, j] f_j  for every row p
+    (StationaryModel.solve, mor/sketched_reductor.py:165-166, over a parameter set; csrc/rom_batch.cu).
+    lhs: Q (r, r) matrices (list or (Q, r, r) tensor); rhs: Pf (r,) vectors (list or (Pf, r) tensor);
+    th (P, Q), tf (P, Pf).  Returns (a (P, r), info (P,) int32): info[p] = i > 0 when U(i, i) of the
+    LU factorisation with partial pivoting is exactly zero, and a_p is then NaN.  With `check`, any
+    such row raises RlaError naming how many failed and the first one (one device-to-host read)."""
+    Q = len(lhs)
+    if Q == 0:
+        raise ValueError("rom_solve_batch: no affine terms")
+    r = int(lhs[0].shape[0])
+    Pf = len(rhs)
+    A = _stack(lhs, (Q, r, r), "rom_solve_batch: lhs")
+    b = _stack(rhs, (Pf, r), "rom_solve_batch: rhs")
+    th = torch.as_tensor(th)
+    P = int(th.shape[0]) if th.dim() == 2 else -1
+    if r < 1 or r > rom_solve_batch_max_r():
+        raise ValueError(f"rom_solve_batch: r={r} outside 1 .. {rom_solve_batch_max_r()}")
+    dev = A.device
+    th, ldth = _param_rows(th, P, Q, "rom_solve_batch: th", dev)
+    tf, ldtf = _param_rows(tf, P, Pf, "rom_solve_batch: tf", dev)
+    a = torch.empty((P, r), dtype=torch.float64, device=dev)
+    info = torch.zeros((P,), dtype=torch.int32, device=dev)
+    if P == 0:
+        return a, info
+    _require_cuda(dev, "rom_solve_batch")
+    A, b = A.to(torch.float64).contiguous(), b.to(device=dev, dtype=torch.float64).contiguous()
+    with torch.cuda.device(dev):
+        _lib.check(lib().rla_rom_solve_batch_f64(A.data_ptr(), Q, r, b.data_ptr() if Pf else None, Pf, th.data_ptr(), ldth,
+                                             tf.data_ptr() if Pf else None, ldtf, P, a.data_ptr(), r, info.data_ptr(),
+                                             stream_ptr()), "rla_rom_solve_batch_f64")
+    if check:
+        bad = info != 0
+        n_bad, first = torch.stack([bad.sum(), torch.argmax(bad.to(torch.int32))]).tolist()
+        if n_bad:
+            raise RlaError(f"rom_solve_batch: {n_bad} of {P} reduced systems are singular "
+                           f"(first: row {first}, U({int(info[first])}, {int(info[first])}) = 0)")
+    return a, info
+
+
+def residual_norm_batch_workspace_bytes(P, kp):
+    """Scratch of residual_norm_batch: one partial sum per row and 128-column tile of the k' sketch."""
+    return int(lib().rla_residual_norm_batch_workspace_bytes(int(P), int(kp)))
+
+
+def residual_norm_batch(W, Q, r, th, tf, a):
+    """est[p] = || sum_q th[p, q] S_q a_p - sum_j tf[p, j] g_j ||_2 for every row p
+    (ResidualErrorEstimator.estimate_error, mor/sketched_reductor.py:216-219, over a parameter set;
+    csrc/rom_batch.cu).  W: (Q r + Pf, k') stack of the (r, k') row blocks S_q^T and the vectors g_j
+    (unit inner stride, any row stride); th (P, Q), tf (P, Pf), a (P, r).  Returns (P,)."""
+    if (not isinstance(W, torch.Tensor) or W.dtype != torch.float64 or W.dim() != 2 or W.shape[0] < Q * r
+            or W.stride(1) != 1):
+        raise ValueError("residual_norm_batch: W must be a 2-D float64 tensor of Q r + Pf rows with unit inner stride")
+    Pf = int(W.shape[0]) - Q * r
+    kp = int(W.shape[1])
+    a = torch.as_tensor(a)
+    P = int(a.shape[0]) if a.dim() == 2 else -1
+    if kp < 1:
+        raise ValueError("residual_norm_batch: empty sketch dimension")
+    dev = W.device
+    a, lda = _param_rows(a, P, r, "residual_norm_batch: a", dev)
+    th, ldth = _param_rows(th, P, Q, "residual_norm_batch: th", dev)
+    tf, ldtf = _param_rows(tf, P, Pf, "residual_norm_batch: tf", dev)
+    est = torch.empty((P,), dtype=torch.float64, device=dev)
+    if P == 0:
+        return est
+    _require_cuda(dev, "residual_norm_batch")
+    ldw = W.stride(0) if W.shape[0] > 1 else kp
+    with torch.cuda.device(dev):
+        ws = dense._workspace(residual_norm_batch_workspace_bytes(P, kp), dev)
+        _lib.check(lib().rla_residual_norm_batch_f64(W.data_ptr(), ldw, Q, r, Pf, kp, th.data_ptr() if Q else None, ldth,
+                                                 tf.data_ptr() if Pf else None, ldtf, a.data_ptr() if r else None, lda,
+                                                 P, est.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr()),
+               "rla_residual_norm_batch_f64")
+    return est

@@ -59,6 +59,14 @@ class AffineModel:
     def thetas(self, mu):
         return ([_coef(c, mu) for c in self.operator_coefficients], [_coef(c, mu) for c in self.rhs_coefficients])
 
+    def thetas_batch(self, mus):
+        """The affine coefficients of every mu, evaluated on the host: float64 arrays (P, Q), (P, Pf)."""
+        Q, Pf = len(self.operator_coefficients), len(self.rhs_coefficients)
+        th, tf = np.empty((len(mus), Q)), np.empty((len(mus), Pf))
+        for p, mu in enumerate(mus):
+            th[p], tf[p] = self.thetas(mu)
+        return th, tf
+
 
 class SketchedReductor:
     def __init__(self, fom, *legacy, embedding_primal=None, embedding_online=None, product=None, inverse_product=None,
@@ -214,6 +222,7 @@ class SketchedRom:
         self.est_lhs_rows, self.est_rhs = est                   # (r, k') row blocks, (k',) vectors
         self.est_lhs = [M.T.contiguous() for M in self.est_lhs_rows]       # k' x r, the reference's orientation
         self.least_squares = least_squares
+        self._lhs_stack = self._rhs_stack = self._est_stack = None         # built by the first batch call
 
     def _thetas(self, theta_lhs, theta_rhs, mu):
         if theta_lhs is None:
@@ -239,6 +248,77 @@ class SketchedRom:
             a = self.solve(theta_lhs, theta_rhs, mu)
         return self.output_functional.T @ a
 
+    # -- the same three over a parameter set: row p of every argument and result belongs to mu_p
+    @property
+    def _dim(self):
+        return self.est_lhs_rows[0].shape[0]                    # (r, k') for both projections
+
+    def _thetas_batch(self, theta_lhs, theta_rhs, mus):
+        """theta_lhs (P, Q) and theta_rhs (P, Pf) as given (the fast path), or fom.thetas of every
+        entry of `mus` stacked on the host and uploaded once."""
+        if mus is not None:
+            if theta_lhs is not None or theta_rhs is not None:
+                raise ValueError("give either mus= or theta_lhs= / theta_rhs=, not both")
+            theta_lhs, theta_rhs = self.fom.thetas_batch(mus)
+        elif theta_lhs is None or theta_rhs is None:
+            raise ValueError("give mus= or both theta_lhs= and theta_rhs=")
+        dev = self.output_functional.device
+        th = torch.as_tensor(theta_lhs, dtype=torch.float64, device=dev)
+        tf = torch.as_tensor(theta_rhs, dtype=torch.float64, device=dev)
+        Q, Pf = len(self.est_lhs_rows), len(self.est_rhs)
+        if th.dim() != 2 or th.shape[1] != Q or tf.dim() != 2 or tf.shape != (th.shape[0], Pf):
+            raise ValueError(f"theta_lhs / theta_rhs: expected shapes (P, {Q}) and (P, {Pf}), "
+                             f"got {tuple(th.shape)} and {tuple(tf.shape)}")
+        return th, tf
+
+    def _batch_a(self, a, th, tf):
+        if a is None:
+            return self.solve_batch(th, tf)
+        a = torch.as_tensor(a, dtype=torch.float64, device=self.output_functional.device)
+        if a.dim() != 2 or a.shape != (th.shape[0], self._dim):
+            raise ValueError(f"a: expected shape ({th.shape[0]}, {self._dim}), got {tuple(a.shape)}")
+        return a
+
+    def solve_batch(self, theta_lhs=None, theta_rhs=None, mus=None, check=True):
+        """Reduced solutions of every mu, (P, r): one launch of the batched LU solve
+        (reductor_ops.rom_solve_batch).  A singular A(mu) raises RlaError naming how many and the
+        first; with check=False its row is NaN instead.  Least-squares (minres) ROMs and r above
+        reductor_ops.rom_solve_batch_max_r() loop over the per-mu `solve`: that path is not accelerated."""
+        th, tf = self._thetas_batch(theta_lhs, theta_rhs, mus)
+        P, r = th.shape[0], self._dim
+        if P == 0:
+            return torch.empty((0, r), dtype=torch.float64, device=th.device)
+        if self.least_squares or r > ops.rom_solve_batch_max_r():
+            return torch.stack([self.solve(th[p], tf[p]) for p in range(P)])
+        if self._lhs_stack is None:
+            self._lhs_stack = torch.stack(self.lhs).contiguous()
+            self._rhs_stack = torch.stack(self.rhs).contiguous() if self.rhs else torch.empty((0, r), dtype=torch.float64,
+                                                                                             device=th.device)
+        return ops.rom_solve_batch(self._lhs_stack, self._rhs_stack, th, tf, check=check)[0]
+
+    def estimate_error_batch(self, a=None, theta_lhs=None, theta_rhs=None, mus=None):
+        """Sketched residual norms of every mu, (P,): one launch of the batched estimator
+        (reductor_ops.residual_norm_batch) for Galerkin and least-squares ROMs alike; `a` (P, r)
+        defaults to solve_batch.  A NaN row of `a` gives NaN."""
+        th, tf = self._thetas_batch(theta_lhs, theta_rhs, mus)
+        a = self._batch_a(a, th, tf)
+        if th.shape[0] == 0:
+            return torch.empty((0,), dtype=torch.float64, device=th.device)
+        if self._est_stack is None:
+            # [S_0^T; ...; S_{Q-1}^T; g_0^T; ...] (N, k'), rows padded to an even length for 16-byte copies
+            kp = self.est_lhs_rows[0].shape[1] if self.est_lhs_rows else self.est_rhs[0].numel()
+            rows = list(self.est_lhs_rows) + [g.reshape(1, -1) for g in self.est_rhs]
+            N = sum(x.shape[0] for x in rows)
+            W = torch.zeros((N, kp + (kp & 1)), dtype=torch.float64, device=th.device)
+            W[:, :kp].copy_(torch.cat(rows, dim=0))
+            self._est_stack = W[:, :kp]
+        return ops.residual_norm_batch(self._est_stack, len(self.est_lhs_rows), self._dim, th, tf, a)
+
+    def output_batch(self, a=None, theta_lhs=None, theta_rhs=None, mus=None):
+        """Outputs of every mu, (P, n_out) = a @ output_functional; `a` defaults to solve_batch."""
+        th, tf = self._thetas_batch(theta_lhs, theta_rhs, mus)
+        return self._batch_a(a, th, tf) @ self.output_functional
+
 
 class EmptyRom:
     """ROM of the empty basis (mor/sketched_reductor.py:189-208)."""
@@ -257,3 +337,26 @@ class EmptyRom:
 
     def output(self, a=None, theta_lhs=None, theta_rhs=None, mu=None):
         return torch.zeros((self.n_out,), dtype=torch.float64, device=self.G.device)
+
+    def _theta_rhs_batch(self, theta_rhs, mus):
+        if mus is not None:
+            theta_rhs = self.fom.thetas_batch(mus)[1]
+        elif theta_rhs is None:
+            raise ValueError("give mus= or theta_rhs=")
+        tf = torch.as_tensor(theta_rhs, dtype=torch.float64, device=self.G.device)
+        if tf.dim() != 2 or tf.shape[1] != self.G.shape[0]:
+            raise ValueError(f"theta_rhs: expected shape (P, {self.G.shape[0]}), got {tuple(tf.shape)}")
+        return tf
+
+    def solve_batch(self, theta_lhs=None, theta_rhs=None, mus=None, check=True):
+        tf = self._theta_rhs_batch(theta_rhs, mus)
+        return torch.empty((tf.shape[0], 0), dtype=torch.float64, device=self.G.device)
+
+    def estimate_error_batch(self, a=None, theta_lhs=None, theta_rhs=None, mus=None):
+        """sqrt(max(tf_p^T G tf_p, 0)) for every row p."""
+        tf = self._theta_rhs_batch(theta_rhs, mus)
+        return torch.sqrt(torch.clamp(((tf @ self.G) * tf).sum(dim=1), min=0.0))
+
+    def output_batch(self, a=None, theta_lhs=None, theta_rhs=None, mus=None):
+        tf = self._theta_rhs_batch(theta_rhs, mus)
+        return torch.zeros((tf.shape[0], self.n_out), dtype=torch.float64, device=self.G.device)
