@@ -372,9 +372,27 @@ int rla_residual_norm_f64(const double *S_dev, int64_t Q, int64_t k, int64_t r,
  * runs on the FP64 tensor pipe with X formed in the kernel; neither X nor the residuals are stored.
  * ws_dev (caller-owned, rla_residual_norm_batch_workspace_bytes(P, kp) = 8 P ceil(kp / 128) bytes)
  * receives the per-tile partial sums, added in tile order: bit-identical from run to run.  A NaN
- * row of a_dev gives a NaN estimate.  Two launches. */
+ * row of a_dev gives a NaN estimate.  Two launches.
+ *
+ * rla_rom_lstsq_batch_f64 replaces, per mu_p, the solve of the least-squares (minres) ROM
+ * (mor/sketched_reductor.py:170-187; LsOperator.apply_inverse, utilities/other_operators.py:12-39):
+ *   a_p = argmin_a || sum_q th[p, q] M_q a - sum_j tf[p, j] g_j ||_2,   M_q: ke x r, g_j: ke.
+ * W_dev (N x ke, row stride ldw, N = Q r + Pf) is the stack [M_0^T; ...; M_{Q-1}^T; g_0^T; ...], the
+ * layout rla_residual_norm_batch_f64 reads (a ROM whose N is below its sketch dimension may pass the
+ * transposed triangular factor of the stack instead: the same minimiser, ke = N).  One CTA per mu
+ * assembles [M(mu) | b(mu)] in panels of rows (ascending q / j, fma), folds each panel into the
+ * r x r triangle by Householder reflections (LAPACK's dlarfg convention) and back-substitutes; row p
+ * of a_dev (row stride lda) receives a_p.  info_dev[p] (int32) = 0, or the first i > 0 with R(i, i)
+ * exactly zero (dtrtrs' convention, as dgels reports it); the row a_p is then NaN.  Results depend on
+ * a mu's own inputs only, not on P: bit-identical from run to run and to a launch with P = 1.
+ * 1 <= r <= rla_rom_lstsq_batch_max_r() (R and one panel in the shared memory of one CTA), ke >= r.
+ * One launch, no workspace. */
 int rla_rom_solve_batch_max_r(void);
 int rla_rom_solve_batch_f64(const double *lhs_dev, int64_t Q, int64_t r, const double *rhs_dev, int64_t Pf,
+                            const double *th_dev, int64_t ldth, const double *tf_dev, int64_t ldtf, int64_t P,
+                            double *a_dev, int64_t lda, int32_t *info_dev, void *stream);
+int rla_rom_lstsq_batch_max_r(void);
+int rla_rom_lstsq_batch_f64(const double *W_dev, int64_t ldw, int64_t Q, int64_t r, int64_t Pf, int64_t k_eff,
                             const double *th_dev, int64_t ldth, const double *tf_dev, int64_t ldtf, int64_t P,
                             double *a_dev, int64_t lda, int32_t *info_dev, void *stream);
 size_t rla_residual_norm_batch_workspace_bytes(int64_t P, int64_t kp);

@@ -76,6 +76,9 @@ _SIGS = {
     "rla_rom_solve_batch_max_r": (c_int, []),
     "rla_rom_solve_batch_f64": (c_int, [_vp, c_int64, c_int64, _vp, c_int64, _vp, c_int64, _vp, c_int64, c_int64,
                                         _vp, c_int64, _vp, _vp]),
+    "rla_rom_lstsq_batch_max_r": (c_int, []),
+    "rla_rom_lstsq_batch_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, c_int64, _vp, c_int64, _vp, c_int64,
+                                        c_int64, _vp, c_int64, _vp, _vp]),
     "rla_residual_norm_batch_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "rla_residual_norm_batch_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, c_int64, _vp, c_int64, _vp,
                                             c_int64, _vp, c_int64, c_int64, _vp, _vp, c_size_t, _vp]),

@@ -15,6 +15,32 @@
 // augmented system must fit the 227 KB of shared memory of one CTA, r (r + 1) 8 bytes:
 // RB_MAX_R = 169.  Threads per CTA from r: 32 up to r = 32, 128 up to 64, 256 beyond.
 //
+// rom_lstsq_batch_kernel: the least-squares (minres) ROM, mor/sketched_reductor.py:170-187 (LsOperator,
+// utilities/other_operators.py:12-39):  a_p = argmin_a || sum_q th[p, q] M_q a - sum_j tf[p, j] g_j ||_2
+// with M_q: k_eff x r, g_j: k_eff, read from the row-major stack W = [M_0^T; ...; g_0^T; ...] (N x k_eff,
+// the residual kernel's layout).  One CTA per mu (grid-stride loop), TSQR in one CTA:
+//   * R (r x r) and the transformed right-hand side d stay in shared memory as [R | d], zero at first;
+//   * rows of [M(mu) | b(mu)] are assembled in panels of c rows straight from W (terms in ascending
+//     q / j, one fma each; W is shared by every mu and stays in L2);
+//   * each panel is folded into [R d; panel] by Householder reflections in LAPACK's dlarfg convention
+//     (beta = -sign(alpha) ||(alpha, x)||, tau = 0 for a zero column), but ||(alpha, x)|| is the plain
+//     sqrt(alpha^2 + sum x_i^2), without dnrm2 / dlapy2 scaling or dlarfg's safmin rescaling: columns
+//     with entries below ~1e-154 underflow (tau = 0, R(j, j) may become an exact zero) and entries
+//     above ~1e154 overflow.  Reflector j touches row j of R and the panel's rows only.  Column k
+//     belongs to the group of G lanes k % (threads / G), whose lanes hold rows lg, lg + G, ...: dot
+//     products are a fixed fma chain per lane and a fixed shuffle tree, and one barrier per
+//     reflector suffices;
+//   * back substitution on d by one warp.
+// Every sum runs in a fixed order and there are no atomics; the configuration depends on r only, so a
+// mu's result depends on its own inputs only (P = 1 and P = 10^5 give the same bits).  info[p] = 0,
+// or the first 1-based i with R(i, i) exactly zero (dtrtrs' convention), and a_p is then NaN.
+// Launch rule (rl_config; threads {64 .. 512} x G {2, 4, 8} x c {32, 64, 128} timed at P = 10^5 on a
+// B200 by tools/sweep_rom_lstsq.py, profiles/rom_lstsq_sweep.jsonl: the fastest at r = 64 and 128,
+// within 12 % of the fastest, 64 threads and G = 8, at r = 16): c = 64 rows per panel; up to r = 32, 64 threads and G = 4; up to 64, 256 threads and G = 8; beyond, 512 threads
+// and G = 8.  Largest r: [R | d] and the panel,
+// r (r + 1) + (r + 1)(c + G) doubles, in 227 KB: RL_MAX_R = 137.  k_eff and Q are limited only by
+// 64-bit indexing.
+//
 // residual_norm_batch_kernel:  est[p] = || sum_q th[p, q] S_q a_p - sum_j tf[p, j] g_j ||_2
 // as one product R(P, k') = X(P, N) W(N, k'), N = Q r + Pf, with
 //   W = [S_0^T; ...; S_{Q-1}^T; g_0^T; ...]   (the ROM's (r, k') row blocks and (k',) vectors)
@@ -112,6 +138,106 @@ __global__ void rom_solve_batch_kernel(const double *__restrict__ lhs, int Q, in
         }
         if (tid == 0) info[p] = inf;
         __syncthreads();                                             // M is reused by the next mu
+    }
+}
+
+// ------------------------------------------------------------------ least-squares solve
+// Shared memory of one CTA: [R | d] (r x (r + 1), row-major) and the panel [Y | y] column-major,
+// column k at Y + k ldy with ldy = c + G (a multiple of 16 plus G: the G-lane groups of a warp
+// read different columns without bank conflicts).
+__host__ __device__ constexpr int64_t rl_smem_doubles(int r, int c, int G) {
+    return (int64_t)r * (r + 1) + (int64_t)(r + 1) * (c + G);
+}
+
+__global__ void __launch_bounds__(512, 2)
+rom_lstsq_batch_kernel(const double *__restrict__ W, int64_t ldw, int Q, int r, int Pf, int64_t ke,
+                       const double *__restrict__ th, int64_t ldth, const double *__restrict__ tf, int64_t ldtf,
+                       int64_t P, double *__restrict__ a, int64_t lda, int32_t *__restrict__ info, int G, int c) {
+    extern __shared__ __align__(16) double rl_smem[];
+    __shared__ double s_tau[2];
+    const int ld = r + 1, ldy = c + G, tid = threadIdx.x, nt = blockDim.x;
+    const int lg = tid & (G - 1), grp = tid / G, ng = nt / G;     // G lanes per column, ng column groups
+    const unsigned gmask = G == 32 ? 0xffffffffu : ((1u << G) - 1u) << ((tid & 31) & ~(G - 1));
+    double *R = rl_smem;                                              // [R | d]
+    double *Y = rl_smem + r * ld;                                     // [Y | y], c x (r + 1)
+    for (int64_t p = blockIdx.x; p < P; p += gridDim.x) {
+        const double *thp = th + p * ldth, *tfp = tf + p * ldtf;
+        for (int e = tid; e < r * ld; e += nt) R[e] = 0.0;
+        for (int64_t i0 = 0; i0 < ke; i0 += c) {
+            // rows i0 .. i0 + cl - 1 of [M(mu) | b(mu)]; consecutive threads read consecutive columns of W
+            const int cl = ke - i0 < c ? (int)(ke - i0) : c;
+            for (int e = tid; e < ld * cl; e += nt) {
+                const int k = e / cl, i = e - k * cl;
+                double s = 0.0;
+                if (k < r)
+                    for (int q = 0; q < Q; ++q) s = fma(__ldg(thp + q), __ldg(W + ((int64_t)q * r + k) * ldw + i0 + i), s);
+                else
+                    for (int j = 0; j < Pf; ++j) s = fma(__ldg(tfp + j), __ldg(W + ((int64_t)Q * r + j) * ldw + i0 + i), s);
+                Y[k * ldy + i] = s;
+            }
+            __syncthreads();
+            // Householder QR of [R d; Y y]: reflector j touches row j of R and the cl panel rows.  Column
+            // k is owned by group k % ng, whose lane lg holds rows lg, lg + G, ...; the group that owns
+            // column j forms reflector j after it has applied reflector j - 1 to it, so one barrier
+            // per reflector orders everything (tau is double-buffered).
+            for (int j = 0; j < r; ++j) {
+                if (grp == j % ng) {                                  // dlarfg on (R(j, j), Y(:, j))
+                    double *v = Y + j * ldy;
+                    double ss = 0.0;
+                    for (int i = lg; i < cl; i += G) ss = fma(v[i], v[i], ss);
+                    for (int off = G >> 1; off; off >>= 1) ss += __shfl_xor_sync(gmask, ss, off);
+                    double tau = 0.0;                                 // zero column: H = I
+                    if (ss != 0.0) {
+                        const double alpha = R[j * ld + j];
+                        const double h = sqrt(fma(alpha, alpha, ss));
+                        const double beta = alpha >= 0.0 ? -h : h;    // beta = -sign(alpha) ||(alpha, x)||
+                        tau = (beta - alpha) / beta;
+                        const double sc = 1.0 / (alpha - beta);
+                        for (int i = lg; i < cl; i += G) v[i] *= sc;
+                        __syncwarp(gmask);                            // every lane has read alpha
+                        if (lg == 0) R[j * ld + j] = beta;
+                    }
+                    if (lg == 0) s_tau[j & 1] = tau;
+                }
+                __syncthreads();
+                const double tau = s_tau[j & 1];
+                if (tau != 0.0) {
+                    const double *v = Y + j * ldy;
+                    for (int k = j + 1 + ((grp - (j + 1) % ng) + ng) % ng; k <= r; k += ng) {
+                        double *y = Y + k * ldy;
+                        const double rjk = R[j * ld + k];
+                        double s = 0.0;
+                        for (int i = lg; i < cl; i += G) s = fma(v[i], y[i], s);
+                        for (int off = G >> 1; off; off >>= 1) s += __shfl_xor_sync(gmask, s, off);
+                        const double w = tau * (rjk + s);
+                        for (int i = lg; i < cl; i += G) y[i] = fma(-w, v[i], y[i]);
+                        __syncwarp(gmask);                            // every lane has read R(j, k)
+                        if (lg == 0) R[j * ld + k] = rjk - w;
+                    }
+                }
+            }
+            __syncthreads();                                          // the next panel overwrites Y
+        }
+        if (tid < 32) {                                               // info, then back substitution
+            int bad = r;
+            for (int i = tid; i < r; i += 32)
+                if (R[i * ld + i] == 0.0) { bad = i; break; }
+#pragma unroll
+            for (int off = 16; off; off >>= 1) bad = min(bad, __shfl_xor_sync(0xffffffffu, bad, off));
+            double *ap = a + p * lda;
+            if (bad < r) {
+                for (int i = tid; i < r; i += 32) ap[i] = __longlong_as_double(0x7ff8000000000000LL);
+            } else {
+                for (int k = r - 1; k >= 0; --k) {
+                    const double x = R[k * ld + r] / R[k * ld + k];
+                    if (tid == 0) ap[k] = x;
+                    for (int i = tid; i < k; i += 32) R[i * ld + r] = fma(-R[i * ld + k], x, R[i * ld + r]);
+                    __syncwarp();
+                }
+            }
+            if (tid == 0) info[p] = bad < r ? bad + 1 : 0;
+        }
+        __syncthreads();                                              // R is reused by the next mu
     }
 }
 
@@ -268,6 +394,21 @@ __global__ void residual_norm_batch_reduce_kernel(const double *__restrict__ ws,
 
 int64_t rn_tiles(int64_t kp) { return (kp + RN_BN - 1) / RN_BN; }
 
+struct RlConfig {
+    int threads, G, c;
+};
+constexpr RlConfig rl_config(int r) {
+    return r <= 32 ? RlConfig{64, 4, 64} : (r <= 64 ? RlConfig{256, 8, 64} : RlConfig{512, 8, 64});
+}
+constexpr int64_t RL_SMEM_LIMIT = 227 * 1024 - 2 * sizeof(double);   // less the static s_tau
+constexpr int rl_max_r() {
+    int r = 1;
+    while (rl_smem_doubles(r + 1, rl_config(r + 1).c, rl_config(r + 1).G) * 8 <= RL_SMEM_LIMIT) ++r;
+    return r;
+}
+constexpr int RL_MAX_R = rl_max_r();
+static_assert(RL_MAX_R >= 128, "the least-squares batch must hold r = 128");
+
 }  // namespace
 }  // namespace rla
 
@@ -294,6 +435,34 @@ extern "C" int rla_rom_solve_batch_f64(const double *lhs_dev, int64_t Q, int64_t
     const int64_t grid = std::min<int64_t>(P, (int64_t)std::max(per_sm, 1) * sm_count());
     rom_solve_batch_kernel<<<(unsigned)grid, threads, smem, (cudaStream_t)stream>>>(
         lhs_dev, (int)Q, (int)r, rhs_dev, (int)Pf, th_dev, ldth, tf_dev, ldtf, P, a_dev, lda, info_dev);
+    count_launch();
+    RLA_CUDA_CHECK(cudaGetLastError());
+    return RLA_OK;
+}
+
+extern "C" int rla_rom_lstsq_batch_max_r(void) { return RL_MAX_R; }
+
+extern "C" int rla_rom_lstsq_batch_f64(const double *W_dev, int64_t ldw, int64_t Q, int64_t r, int64_t Pf, int64_t ke,
+                                       const double *th_dev, int64_t ldth, const double *tf_dev, int64_t ldtf, int64_t P,
+                                       double *a_dev, int64_t lda, int32_t *info_dev, void *stream) {
+    RLA_REQUIRE(Q >= 0 && Pf >= 0 && P >= 0 && r >= 1 && ke >= 1 && ldw >= ke && ldth >= Q && ldtf >= Pf && lda >= r,
+                "rla_rom_lstsq_batch_f64: bad sizes");
+    RLA_REQUIRE(r <= RL_MAX_R, "rla_rom_lstsq_batch_f64: r=%lld exceeds the largest supported r=%d",
+                (long long)r, RL_MAX_R);
+    RLA_REQUIRE(ke >= r, "rla_rom_lstsq_batch_f64: k_eff=%lld < r=%lld: the system is underdetermined",
+                (long long)ke, (long long)r);
+    RLA_REQUIRE(Q < (1 << 30) && Pf < (1 << 30), "rla_rom_lstsq_batch_f64: too many affine terms");
+    if (P == 0) return RLA_OK;
+    RLA_REQUIRE(a_dev && info_dev && W_dev && (Q == 0 || th_dev) && (Pf == 0 || tf_dev),
+                "rla_rom_lstsq_batch_f64: null pointer");
+    const RlConfig cfg = rl_config((int)r);
+    const int smem = (int)(rl_smem_doubles((int)r, cfg.c, cfg.G) * sizeof(double));
+    RLA_CUDA_CHECK(cudaFuncSetAttribute(rom_lstsq_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    int per_sm = 0;
+    RLA_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rom_lstsq_batch_kernel, cfg.threads, smem));
+    const int64_t grid = std::min<int64_t>(P, (int64_t)std::max(per_sm, 1) * sm_count());
+    rom_lstsq_batch_kernel<<<(unsigned)grid, cfg.threads, smem, (cudaStream_t)stream>>>(
+        W_dev, ldw, (int)Q, (int)r, (int)Pf, ke, th_dev, ldth, tf_dev, ldtf, P, a_dev, lda, info_dev, cfg.G, cfg.c);
     count_launch();
     RLA_CUDA_CHECK(cudaGetLastError());
     return RLA_OK;

@@ -295,6 +295,54 @@ def rom_solve_batch(lhs, rhs, th, tf, check=True):
     return a, info
 
 
+def rom_lstsq_batch_max_r():
+    """Largest reduced dimension r of rom_lstsq_batch (R and one row panel in one CTA's shared memory)."""
+    return int(lib().rla_rom_lstsq_batch_max_r())
+
+
+def rom_lstsq_batch(W, Q, r, th, tf, check=True):
+    """Reduced least-squares solves  a_p = argmin_a || sum_q th[p, q] M_q a - sum_j tf[p, j] g_j ||_2
+    for every row p (the minres ROM's LsOperator solve, mor/sketched_reductor.py:170-187, over a
+    parameter set; csrc/rom_batch.cu).  W: (Q r + Pf, k_eff) stack [M_0^T; ...; M_{Q-1}^T; g_0^T; ...]
+    of the (k_eff, r) matrices M_q and (k_eff,) vectors g_j (unit inner stride, any row stride), with
+    k_eff >= r; th (P, Q), tf (P, Pf).  Returns (a (P, r), info (P,) int32): info[p] = i > 0 when
+    R(i, i) of the Householder QR is exactly zero, and a_p is then NaN.  With `check`, any such row
+    raises RlaError naming how many failed and the first one (one device-to-host read)."""
+    if (not isinstance(W, torch.Tensor) or W.dtype != torch.float64 or W.dim() != 2 or W.shape[0] < Q * r
+            or (W.shape[1] > 1 and W.stride(1) != 1)):
+        raise ValueError("rom_lstsq_batch: W must be a 2-D float64 tensor of Q r + Pf rows with unit inner stride")
+    if Q < 1:
+        raise ValueError("rom_lstsq_batch: no affine terms")
+    if r < 1 or r > rom_lstsq_batch_max_r():
+        raise ValueError(f"rom_lstsq_batch: r={r} outside 1 .. {rom_lstsq_batch_max_r()}")
+    Pf, ke = int(W.shape[0]) - Q * r, int(W.shape[1])
+    if ke < r:
+        raise ValueError(f"rom_lstsq_batch: k_eff={ke} < r={r}: the reduced systems are underdetermined")
+    th = torch.as_tensor(th)
+    P = int(th.shape[0]) if th.dim() == 2 else -1
+    dev = W.device
+    th, ldth = _param_rows(th, P, Q, "rom_lstsq_batch: th", dev)
+    tf, ldtf = _param_rows(tf, P, Pf, "rom_lstsq_batch: tf", dev)
+    a = torch.empty((P, r), dtype=torch.float64, device=dev)
+    info = torch.zeros((P,), dtype=torch.int32, device=dev)
+    if P == 0:
+        return a, info
+    _require_cuda(dev, "rom_lstsq_batch")
+    ldw = W.stride(0) if W.shape[0] > 1 else ke
+    with torch.cuda.device(dev):
+        _lib.check(lib().rla_rom_lstsq_batch_f64(W.data_ptr(), ldw, Q, r, Pf, ke, th.data_ptr(), ldth,
+                                             tf.data_ptr() if Pf else None, ldtf, P, a.data_ptr(), r,
+                                             info.data_ptr(), stream_ptr()), "rla_rom_lstsq_batch_f64")
+    if check:
+        bad = info != 0
+        first = torch.argmax(bad.to(torch.int32))
+        n_bad, first, i = torch.stack([bad.sum(), first, info[first].to(torch.int64)]).tolist()
+        if n_bad:
+            raise RlaError(f"rom_lstsq_batch: {n_bad} of {P} reduced systems are rank-deficient "
+                           f"(first: row {first}, R({i}, {i}) = 0)")
+    return a, info
+
+
 def residual_norm_batch_workspace_bytes(P, kp):
     """Scratch of residual_norm_batch: one partial sum per row and 128-column tile of the k' sketch."""
     return int(lib().rla_residual_norm_batch_workspace_bytes(int(P), int(kp)))

@@ -223,14 +223,40 @@ class SketchedRom:
         self.est_lhs = [M.T.contiguous() for M in self.est_lhs_rows]       # k' x r, the reference's orientation
         self.least_squares = least_squares
         self._lhs_stack = self._rhs_stack = self._est_stack = None         # built by the first batch call
+        self._ls_stack = None                                              # built by the first least-squares solve
 
     def _thetas(self, theta_lhs, theta_rhs, mu):
         if theta_lhs is None:
             theta_lhs, theta_rhs = self.fom.thetas(mu)
         return theta_lhs, theta_rhs
 
+    def _lstsq_on_device(self):
+        """Whether the least-squares solves take the batched QR kernel: r within its shared-memory
+        limit and at least r rows (k' >= r; the stack has N = Q r + Pf >= r rows otherwise)."""
+        return self._dim <= ops.rom_lstsq_batch_max_r() and self.lhs[0].shape[0] >= self._dim
+
+    def _lstsq_stack(self):
+        """The (N, k_eff) stack [M_0^T; ...; M_{Q-1}^T; g_0^T; ...] that reductor_ops.rom_lstsq_batch
+        reads, built once.  When N = Q r + Pf is below k', the k' x N matrix Wc = [M_0 ... g_0 ...] is
+        replaced by its triangular factor R (Wc = Q R, the stack becomes R^T, k_eff = N): ||Wc x|| =
+        ||R x|| for every x, so every mu has the same minimiser, and the per-mu work no longer grows
+        with k'."""
+        if self._ls_stack is None:
+            Wc = torch.cat(list(self.lhs) + [v.reshape(-1, 1) for v in self.rhs], dim=1)
+            if Wc.shape[1] < Wc.shape[0]:
+                Wc = torch.linalg.qr(Wc, mode="r").R
+            self._ls_stack = Wc.T.contiguous()
+        return self._ls_stack
+
     def solve(self, theta_lhs=None, theta_rhs=None, mu=None):
+        """The reduced solution of one mu.  A least-squares ROM within the batched kernel's envelope
+        solves it as solve_batch does (P = 1, the same bits); a rank-deficient A(mu) raises RlaError."""
         theta_lhs, theta_rhs = self._thetas(theta_lhs, theta_rhs, mu)
+        if self.least_squares and self._lstsq_on_device():
+            dev = self.output_functional.device
+            th = torch.as_tensor(theta_lhs, dtype=torch.float64, device=dev).reshape(1, -1)
+            tf = torch.as_tensor(theta_rhs, dtype=torch.float64, device=dev).reshape(1, -1)
+            return ops.rom_lstsq_batch(self._lstsq_stack(), len(self.lhs), self._dim, th, tf)[0][0]
         A = sum(t * M for t, M in zip(theta_lhs, self.lhs))
         b = sum(t * v for t, v in zip(theta_rhs, self.rhs))
         if self.least_squares:                                   # LsOperator: apply_inverse(least_squares=True)
@@ -281,13 +307,18 @@ class SketchedRom:
 
     def solve_batch(self, theta_lhs=None, theta_rhs=None, mus=None, check=True):
         """Reduced solutions of every mu, (P, r): one launch of the batched LU solve
-        (reductor_ops.rom_solve_batch).  A singular A(mu) raises RlaError naming how many and the
-        first; with check=False its row is NaN instead.  Least-squares (minres) ROMs and r above
-        reductor_ops.rom_solve_batch_max_r() loop over the per-mu `solve`: that path is not accelerated."""
+        (reductor_ops.rom_solve_batch) for a Galerkin ROM, of the batched Householder QR solve
+        (reductor_ops.rom_lstsq_batch) for a least-squares (minres) ROM.  A singular or rank-deficient
+        A(mu) raises RlaError naming how many and the first; with check=False its row is NaN instead.
+        Outside the kernels' envelopes (Galerkin: r above rom_solve_batch_max_r(); least squares: r
+        above rom_lstsq_batch_max_r() or k' < r) the per-mu `solve` runs in a loop, which is not
+        accelerated."""
         th, tf = self._thetas_batch(theta_lhs, theta_rhs, mus)
         P, r = th.shape[0], self._dim
         if P == 0:
             return torch.empty((0, r), dtype=torch.float64, device=th.device)
+        if self.least_squares and self._lstsq_on_device():
+            return ops.rom_lstsq_batch(self._lstsq_stack(), len(self.lhs), r, th, tf, check=check)[0]
         if self.least_squares or r > ops.rom_solve_batch_max_r():
             return torch.stack([self.solve(th[p], tf[p]) for p in range(P)])
         if self._lhs_stack is None:
