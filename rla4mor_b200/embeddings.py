@@ -31,6 +31,16 @@ One option is new: `options['rng']`
     two-part split of the block and FP64 accumulation of 64-term partial sums,
     csrc/gemm32.cu: 1e-5 relative, ~4x the FP64 path); FP64 blocks use the same Theta.
 SRHT signs and row indices are always the reference's NumPy draws (bit-exact).
+
+The two Gaussian classes share one model of Theta, a table of row blocks: block b is rows
+0 .. size_b - 1 of the stream of seed_b.  A `BlockGaussianEmbedding` lists its blocks; a
+`GaussianEmbedding` is the table of one block (its seed, k rows), so every way of producing Theta,
+`apply` and `apply_adjoint` are written once for both.  Theta is real, so a complex block is
+sketched (and taken through the adjoint) as its real and imaginary parts; that needs an identity
+`sqrt_product`, otherwise `TypeError`, as for the SRHT.  `apply_adjoint` multiplies by
+`get_matrix_device()` when a Theta or matrix is already on the device (a `GaussianEmbedding` in
+'mt19937' always holds its draw there); otherwise the Philox modes run one kernel over all blocks
+with Theta generated inside it, and 'mt19937' draws one block at a time and accumulates.
 """
 import logging
 
@@ -238,6 +248,27 @@ class RandomEmbedding:
         for name in self._init_args:
             setattr(self, "_arg_" + name, loc[name])
 
+    def _init(self, args, seeded=True):
+        """The constructor body of the embeddings (embeddings.py:132-141 and the like): the argument
+        record `with_` uses, with default options and, if `seeded`, a random seed filled in; frozen
+        options; Q, the identity by default; the spaces; empty caches."""
+        args = dict(args)
+        if args["options"] is None:
+            args["options"] = dict()
+        if seeded and args["_seed"] is None:
+            args["_seed"] = np.random.randint(0, high=2 ** 32 - 1)
+        self._store_args(args)
+        self._seed = args["_seed"]
+        self.options = FrozenDict(args["options"])
+        sqrt_product = args["sqrt_product"]
+        self.sqrt_product = IdentityOperator(args["source"]) if sqrt_product is None else sqrt_product
+        self.source = self.sqrt_product.source
+        self.range_id = args["range_id"]
+        self.range = DeviceVectorSpace(self.compute_dim(), id=self.range_id)
+        self._matrix = None
+        self._matrix_dev = None
+        self._random_matrix = None
+
     def _apply_sqrt_product(self, U):
         """Q U as a CUDA block, plus the kind of the caller's container."""
         if isinstance(U, DeviceVectorArray):
@@ -255,34 +286,6 @@ class RandomEmbedding:
         if isinstance(Q, IdentityOperator):
             return rmat
         return Q.apply_adjoint(Q.range.from_numpy(rmat.conj())).to_numpy().conj()
-
-    def _gaussian_adjoint(self, U, product, includes_sqrt_product=False):
-        """V @ get_matrix() of the Gaussian embeddings from `product(v)`, a real CUDA block times
-        the (k, n) matrix: Theta, then Q^H applied here, or the explicit matrix that already holds it
-        (`includes_sqrt_product`).  Theta is real, so a complex block goes through as its real and
-        imaginary parts; that needs an identity sqrt_product, as SrhtEmbedding.apply_adjoint does."""
-        torch = require_cuda()
-        if isinstance(U, DeviceVectorArray):
-            assert U in self.range
-        v, kind = _unwrap(U)
-        assert v.shape[1] == self.range.dim
-        Q = self.sqrt_product
-        if v.is_complex():
-            if not isinstance(Q, IdentityOperator):
-                raise TypeError(f"{type(self).__name__}.apply_adjoint: complex blocks need an identity sqrt_product")
-            m = v.shape[0]
-            w2 = product(torch.cat([v.real, v.imag], dim=0).to(torch.float64))
-            return _wrap_result(kind, self.source, torch.complex(w2[:m], w2[m:]))
-        w = product(v.to(torch.float64))
-        if not includes_sqrt_product and not isinstance(Q, IdentityOperator):
-            w = Q.apply_adjoint(DeviceVectorArray(Q.range, w)).data
-        return _wrap_result(kind, self.source, w)
-
-    @property
-    def _rng_mode(self):
-        mode = self.options.get("rng", "mt19937")
-        assert mode in ("mt19937", "philox", "philox_rademacher", "philox_tf32"), f"unknown options['rng'] = {mode!r}"
-        return mode
 
 
 def _gaussian_dim(opt):
@@ -306,20 +309,7 @@ class SrhtEmbedding(RandomEmbedding):
 
     def __init__(self, source=None, sqrt_product=None, options=None, range_id=None, _seed=None):
         assert not (source is None) or not (sqrt_product is None)          # :131
-        if options is None:
-            options = dict()
-        if _seed is None:
-            _seed = np.random.randint(0, high=2 ** 32 - 1)
-        self._store_args(locals())
-        self._seed = _seed
-        self.options = FrozenDict(options)
-        self.sqrt_product = IdentityOperator(source) if sqrt_product is None else sqrt_product
-        self.source = self.sqrt_product.source
-        self.range_id = range_id
-        self.range = DeviceVectorSpace(self.compute_dim(), id=range_id)
-        self._matrix = None
-        self._matrix_dev = None
-        self._random_matrix = None
+        self._init(locals())
         self._plans = {}
         self._order_dev = None
 
@@ -452,37 +442,24 @@ class SrhtEmbedding(RandomEmbedding):
         return out
 
 
-class GaussianEmbedding(RandomEmbedding):
-    """rla/embeddings.py:214-270."""
+class _GaussianBase(RandomEmbedding):
+    """What GaussianEmbedding and BlockGaussianEmbedding share: Theta as a table of row blocks.  Block b
+    is rows 0 .. size_b - 1 of the stream of seed_b (`_block_seeds`, `_block_sizes`), scaled by
+    1/sqrt(k): NumPy's RandomState(seed_b).normal draw in 'mt19937', the kernels' generator
+    g(seed_b, row, col) in the Philox modes.  A GaussianEmbedding is the table of one block."""
+    # GaussianEmbedding keeps its 'mt19937' draw on the device in `_theta_dev`; the block embedding
+    # draws Theta again on every use, as the reference does (:430,452-461)
+    _keeps_theta = False
+    _theta_dev = None
 
-    def __init__(self, source=None, sqrt_product=None, options=None, range_id=None, _seed=None):
-        assert not (source is None) or not (sqrt_product is None)          # :219
-        if options is None:
-            options = dict()
-        if _seed is None:
-            _seed = np.random.randint(0, high=2 ** 32 - 1)
-        self._store_args(locals())
-        self._seed = _seed
-        self.options = FrozenDict(options)
-        self.sqrt_product = IdentityOperator(source) if sqrt_product is None else sqrt_product
-        self.source = self.sqrt_product.source
-        self.range_id = range_id
-        self.range = DeviceVectorSpace(self.compute_dim(), id=range_id)
-        self._matrix = None
-        self._matrix_dev = None
-        self._theta_dev = None
-        # the reference draws Theta eagerly (:230); on-the-fly modes never hold it
-        self._random_matrix = self._compute_random_matrix() if self._rng_mode == "mt19937" else None
-
-    def compute_dim(self):                                                 # :234-247
+    def compute_dim(self):                                                 # :234-247, :409-422
         return _gaussian_dim(self.options)
 
-    def update(self):
-        self._theta_dev = None
-        if self._rng_mode == "mt19937":
-            self._random_matrix = self._compute_random_matrix()
-        if not (self._matrix is None):
-            self._matrix = self._compute_matrix()
+    @property
+    def _rng_mode(self):
+        mode = self.options.get("rng", "mt19937")
+        assert mode in ("mt19937", "philox", "philox_rademacher", "philox_tf32"), f"unknown options['rng'] = {mode!r}"
+        return mode
 
     def _kind(self):
         return {"philox_rademacher": dense.KIND_RADEMACHER, "philox_tf32": dense.KIND_NORMAL_TF32}.get(
@@ -492,73 +469,189 @@ class GaussianEmbedding(RandomEmbedding):
         """Theta exact in TF32: float32 blocks can stay float32 (tcgen05 path, csrc/gemm32.cu)."""
         return self._rng_mode in ("philox_rademacher", "philox_tf32")
 
-    def apply(self, U, mu=None):                                           # :250-254
+    @property
+    def _scale(self):
+        return 1.0 / np.sqrt(self.range.dim)
+
+    def _table(self, blocks=None):
+        """(seeds, sizes) of the listed blocks, all by default."""
+        seeds, sizes = self._block_seeds, self._block_sizes
+        if blocks is None:
+            return seeds, sizes
+        return [seeds[i] for i in blocks], [sizes[i] for i in blocks]
+
+    # -- Theta
+    def _theta_device(self, blocks=None, plan=None):
+        """The stacked rows of the listed blocks (all by default) as a CUDA tensor.  'mt19937': NumPy's
+        draw made on the device (csrc/mt19937.cu); given `plan`, a NormalPlan over the streams of the
+        whole table, the one listed block is drawn from it.  Philox modes: what the kernels generate."""
         torch = require_cuda()
-        k = self.range.dim
-        if _is_host_tensor(U) and isinstance(self.sqrt_product, IdentityOperator):
-            # block in host memory: streamed by column slabs (on-the-fly Theta: accumulate per
-            # slab at full GEMM height) or by groups of vectors (explicit Theta)
-            from .streaming import apply_streamed, apply_streamed_rng
-            assert U.shape[1] == self.source.dim
-            if self._rng_mode == "mt19937" or not (U.dtype == torch.float64 or (U.dtype == torch.float32 and self._tf32_ok())):
-                return apply_streamed(self.apply, U, k, return_host=True)
-            return apply_streamed_rng(self._seed, self._kind(), 1.0 / np.sqrt(k), k, U, return_host=True)
-        qu, kind = self._apply_sqrt_product(U)
-        if qu.is_complex():                                                # Theta is real: sketch both parts in one pass
-            m = qu.shape[0]
-            y2 = self.apply(torch.cat([qu.real, qu.imag], dim=0).to(torch.float64).contiguous()) \
-                if isinstance(self.sqrt_product, IdentityOperator) else None
-            if y2 is None:
-                raise TypeError("GaussianEmbedding.apply: complex blocks need an identity sqrt_product")
-            return _wrap_result(kind, self.range, torch.complex(y2[:m], y2[m:]))
-        if qu.dtype != torch.float64 and not (qu.dtype == torch.float32 and self._tf32_ok()):
-            qu = qu.to(torch.float64)
-        if self._rng_mode == "mt19937":
-            if self._theta_dev is None or self._theta_dev.device != qu.device:
-                self._theta_dev = torch.from_numpy(self._random_matrix).to(qu.device)
-            y = dense.gauss_apply_explicit(self._theta_dev, qu)
-        else:
-            y = dense.embed_apply_rng(self._seed, self._kind(), 1.0 / np.sqrt(k), k, qu)
-        return _wrap_result(kind, self.range, y)
-
-    def apply_adjoint(self, U, mu=None):
-        """V @ get_matrix()  (pyMOR's generic adjoint of a matrix operator).  'mt19937', or a matrix
-        already on the device: the product with that matrix.  Otherwise V Theta with Theta generated
-        in the kernel (csrc/adjoint_rng.cu), then Q^H: Theta is neither materialised nor kept."""
-        if self._rng_mode == "mt19937" or self._matrix_dev is not None:
-            from .reductor_ops import gemm_nn
-            return self._gaussian_adjoint(U, lambda v: gemm_nn(v, self.get_matrix_device()), includes_sqrt_product=True)
-        k = self.range.dim
+        seeds, sizes = self._table(blocks)
         n = self.sqrt_product.range.dim
-        return self._gaussian_adjoint(
-            U, lambda v: dense.embed_adjoint_rng([self._seed], [0, k], self._kind(), 1.0 / np.sqrt(k), v, n))
+        if self._rng_mode != "mt19937":
+            parts = [dense.theta_materialize(s, self._kind(), self._scale, b, n) for s, b in zip(seeds, sizes)]
+            return parts[0] if len(parts) == 1 else torch.cat(parts, dim=0)
+        if self._keeps_theta:
+            if self._theta_dev is None:
+                self._theta_dev = mt19937.gaussian_matrix(seeds, sizes, n, self._scale)
+            return self._theta_dev
+        if plan is None:
+            return mt19937.gaussian_matrix(seeds, sizes, n, self._scale)
+        (i,), (b,) = blocks, sizes
+        theta = torch.empty((b, n), dtype=torch.float64, device=plan.device)
+        count = np.zeros(len(plan.counts), np.int64)
+        count[i] = b * n
+        if theta.numel():
+            plan.execute(theta.view(-1), 0, count, 0, self._scale)
+        return theta
 
-    def _compute_matrix(self):                                             # :258-262
+    def _theta_host(self, blocks=None):
+        """The same rows as a NumPy array.  'mt19937' is drawn by NumPy itself only where there is no
+        CUDA device (an embedding built on the host); otherwise the device draw is downloaded, in
+        bounded chunks unless it is kept anyway."""
+        seeds, sizes = self._table(blocks)
+        n = self.sqrt_product.range.dim
+        if self._rng_mode == "mt19937" and not _cuda_available():
+            return np.vstack([np.random.RandomState(s).normal(size=(b, n), loc=0, scale=self._scale)
+                              for s, b in zip(seeds, sizes)])
+        if self._rng_mode == "mt19937" and not self._keeps_theta:
+            return mt19937.gaussian_matrix_host(seeds, sizes, n, self._scale)
+        return self._theta_device(blocks).cpu().numpy()
+
+    def _compute_random_matrix(self):                                      # :265-270, :444-450
+        return self._theta_host()
+
+    def _compute_random_matrix_device(self):
+        return self._theta_device()
+
+    def _compute_matrix(self):                                             # :258-262, :437-441
         gauss = self._random_matrix if self._random_matrix is not None else self._compute_random_matrix()
         return self._adjoint_sqrt_product(gauss)
 
-    def _compute_random_matrix(self):                                      # :265-270
-        k = self.range.dim
-        n = self.sqrt_product.range.dim
-        seed = self._seed
-        if self._rng_mode == "mt19937":
-            if not _cuda_available():
-                return np.random.RandomState(seed).normal(size=(k, n), loc=0, scale=1 / np.sqrt(k))
-            # the device draw is kept: apply() and get_matrix_device() use it without an upload
-            self._theta_dev = mt19937.gaussian_matrix([seed], [k], n, 1 / np.sqrt(k))
-            return self._theta_dev.cpu().numpy()
-        return dense.theta_materialize(seed, self._kind(), 1.0 / np.sqrt(k), k, n).cpu().numpy()
+    def update(self):
+        self._theta_dev = None
+        super().update()
 
-    def _compute_random_matrix_device(self):
+    # -- the operator
+    def apply(self, U, mu=None):                                           # :250-254, :425-434
         torch = require_cuda()
-        k = self.range.dim
+        qu, kind = self._apply_sqrt_product(U)
+        if qu.is_complex():                                                # Theta is real: sketch both parts in one pass
+            if not isinstance(self.sqrt_product, IdentityOperator):
+                raise TypeError(f"{type(self).__name__}.apply: complex blocks need an identity sqrt_product")
+            m = qu.shape[0]
+            y2 = self.sketch_blocks(torch.cat([qu.real, qu.imag], dim=0).to(torch.float64).contiguous())
+            return _wrap_result(kind, self.range, torch.complex(y2[:m], y2[m:]))
+        if qu.dtype != torch.float64 and not (qu.dtype == torch.float32 and self._tf32_ok()):
+            qu = qu.to(torch.float64)
+        return _wrap_result(kind, self.range, self.sketch_blocks(qu))
+
+    def sketch_blocks(self, V, blocks=None):
+        """Sketch of the real CUDA block V (m, n), already Q U, by the listed row blocks of Theta (all by
+        default), their columns side by side: `apply`'s result, or its columns of those blocks.  V is
+        float64, or float32 where `_tf32_ok()`."""
+        torch = require_cuda()
+        seeds, sizes = self._block_seeds, self._block_sizes
+        blocks = range(len(sizes)) if blocks is None else blocks
+        plan = None
+        if self._rng_mode == "mt19937" and not self._keeps_theta and len(blocks):
+            # one plan (jump-ahead + acceptance count) for the streams of all blocks
+            plan = mt19937.NormalPlan(seeds, [b * self.sqrt_product.range.dim for b in sizes], V.device)
+
+        def sketch(i):                                                     # :430-432
+            if self._rng_mode == "mt19937":
+                return dense.gauss_apply_explicit(self._theta_device([i], plan).to(V.device), V)
+            return dense.embed_apply_rng(seeds[i], self._kind(), self._scale, sizes[i], V)
+
+        if len(blocks) == 1:
+            return sketch(blocks[0])
+        out = torch.empty((V.shape[0], sum(sizes[i] for i in blocks)), dtype=torch.float64, device=V.device)
+        off = 0
+        for i in blocks:
+            out[:, off:off + sizes[i]].copy_(sketch(i))
+            off += sizes[i]
+        return out
+
+    def apply_adjoint(self, U, mu=None):
+        """V @ get_matrix()  (pyMOR's adjoint of the explicit matrix).  With a Theta or matrix already on
+        the device: the product with get_matrix_device().  Otherwise V Theta, then Q^H: in the Philox
+        modes one launch over all blocks with Theta generated in the kernel (csrc/adjoint_rng.cu); in
+        'mt19937' one plan for all blocks, each block drawn in turn and V[:, block] Theta_b accumulated,
+        so one block of Theta is held at a time."""
+        from .reductor_ops import gemm_nn
+        if self._theta_dev is not None or self._matrix_dev is not None:
+            return self._gaussian_adjoint(U, lambda v: gemm_nn(v, self.get_matrix_device()), includes_sqrt_product=True)
+        seeds, sizes = self._block_seeds, self._block_sizes
         n = self.sqrt_product.range.dim
+        if self._rng_mode != "mt19937":
+            starts = np.concatenate([[0], np.cumsum(sizes)])
+            return self._gaussian_adjoint(
+                U, lambda v: dense.embed_adjoint_rng(seeds, starts, self._kind(), self._scale, v, n))
+
+        def product(v):
+            plan = mt19937.NormalPlan(seeds, [b * n for b in sizes], v.device)
+            out, off = None, 0
+            for i, b in enumerate(sizes):
+                w = gemm_nn(v[:, off:off + b], self._theta_device([i], plan))
+                out = w if out is None else out.add_(w)
+                off += b
+            return out
+        return self._gaussian_adjoint(U, product)
+
+    def _gaussian_adjoint(self, U, product, includes_sqrt_product=False):
+        """V @ get_matrix() from `product(v)`, a real CUDA block times the (k, n) matrix: Theta, then
+        Q^H applied here, or the explicit matrix that already holds it (`includes_sqrt_product`).  Theta
+        is real, so a complex block goes through as its real and imaginary parts; that needs an identity
+        sqrt_product, as SrhtEmbedding.apply_adjoint does."""
+        torch = require_cuda()
+        if isinstance(U, DeviceVectorArray):
+            assert U in self.range
+        v, kind = _unwrap(U)
+        assert v.shape[1] == self.range.dim
+        Q = self.sqrt_product
+        if v.is_complex():
+            if not isinstance(Q, IdentityOperator):
+                raise TypeError(f"{type(self).__name__}.apply_adjoint: complex blocks need an identity sqrt_product")
+            m = v.shape[0]
+            w2 = product(torch.cat([v.real, v.imag], dim=0).to(torch.float64))
+            return _wrap_result(kind, self.source, torch.complex(w2[:m], w2[m:]))
+        w = product(v.to(torch.float64))
+        if not includes_sqrt_product and not isinstance(Q, IdentityOperator):
+            w = Q.apply_adjoint(DeviceVectorArray(Q.range, w)).data
+        return _wrap_result(kind, self.source, w)
+
+
+class GaussianEmbedding(_GaussianBase):
+    """rla/embeddings.py:214-270: the table of one block, its seed and k rows."""
+    _keeps_theta = True
+
+    def __init__(self, source=None, sqrt_product=None, options=None, range_id=None, _seed=None):
+        assert not (source is None) or not (sqrt_product is None)          # :219
+        self._init(locals())
+        # the reference draws Theta eagerly (:230); on-the-fly modes never hold it
         if self._rng_mode == "mt19937":
-            # NumPy's MT19937 draw made on the device; shared with apply()
-            if self._theta_dev is None:
-                self._theta_dev = mt19937.gaussian_matrix([self._seed], [k], n, 1 / np.sqrt(k))
-            return self._theta_dev
-        return dense.theta_materialize(self._seed, self._kind(), 1.0 / np.sqrt(k), k, n)
+            self._random_matrix = self._compute_random_matrix()
+
+    @property
+    def _block_seeds(self):
+        return [self._seed]
+
+    @property
+    def _block_sizes(self):
+        return [self.range.dim]
+
+    def apply(self, U, mu=None):                                           # :250-254
+        if _is_host_tensor(U) and isinstance(self.sqrt_product, IdentityOperator):
+            # block in host memory: streamed by column slabs (on-the-fly Theta: accumulate per
+            # slab at full GEMM height) or by groups of vectors (explicit Theta)
+            torch = require_cuda()
+            from .streaming import apply_streamed, apply_streamed_rng
+            assert U.shape[1] == self.source.dim
+            k = self.range.dim
+            if self._rng_mode == "mt19937" or not (U.dtype == torch.float64 or (U.dtype == torch.float32 and self._tf32_ok())):
+                return apply_streamed(self.apply, U, k, return_host=True)
+            return apply_streamed_rng(self._seed, self._kind(), self._scale, k, U, return_host=True)
+        return super().apply(U, mu)
 
 
 class IdentityEmbedding(RandomEmbedding):
@@ -566,17 +659,7 @@ class IdentityEmbedding(RandomEmbedding):
 
     def __init__(self, source=None, sqrt_product=None, options=None, range_id=None, _seed=None):
         assert not (source is None) or not (sqrt_product is None)          # :279
-        if options is None:
-            options = dict()
-        self._store_args(locals())
-        self._seed = _seed
-        self.options = FrozenDict(options)
-        self.sqrt_product = IdentityOperator(source) if sqrt_product is None else sqrt_product
-        self.source = self.sqrt_product.source
-        self.range_id = range_id
-        self.range = DeviceVectorSpace(self.compute_dim(), id=range_id)
-        self._matrix = None
-        self._matrix_dev = None
+        self._init(locals(), seeded=False)
         self._random_matrix = self._compute_random_matrix()
 
     def compute_dim(self):                                                 # :291-292
@@ -653,25 +736,14 @@ class EmbeddingVectorized(RandomEmbedding):
         return self.embedding._compute_random_matrix()
 
 
-class BlockGaussianEmbedding(RandomEmbedding):
+class BlockGaussianEmbedding(_GaussianBase):
     """rla/embeddings.py:373-467: Theta in row blocks of at most `max_block_size`
     rows, one seed per block."""
 
     def __init__(self, source=None, sqrt_product=None, options=None, range_id=None, _seed=None):
         assert not (source is None) or not (sqrt_product is None)          # :378
         assert options is not None and "max_block_size" in options.keys()  # :379
-        if _seed is None:
-            _seed = np.random.randint(0, high=2 ** 32 - 1)
-        self._store_args(locals())
-        self._seed = _seed
-        self.options = FrozenDict(options)
-        self.sqrt_product = IdentityOperator(source) if sqrt_product is None else sqrt_product
-        self.source = self.sqrt_product.source
-        self.range_id = range_id
-        self.range = DeviceVectorSpace(self.compute_dim(), id=range_id)
-        self._matrix = None
-        self._matrix_dev = None
-        self._random_matrix = None
+        self._init(locals())
         # block sizes (:393-400)
         max_block_size = options.get("max_block_size")
         m = self.range.dim // max_block_size
@@ -688,130 +760,20 @@ class BlockGaussianEmbedding(RandomEmbedding):
             block_seeds = np.random.RandomState(self._seed).randint(0, 2 ** 32 - 1, size=len(block_sizes))
         self.block_seeds = block_seeds
 
-    def compute_dim(self):                                                 # :409-422
-        return _gaussian_dim(self.options)
+    @property
+    def _block_seeds(self):
+        return [int(s) for s in self.block_seeds]
 
-    def update(self):
-        if not (self._matrix is None):
-            self._matrix = self._compute_matrix()
-
-    def _kind(self):
-        return {"philox_rademacher": dense.KIND_RADEMACHER, "philox_tf32": dense.KIND_NORMAL_TF32}.get(
-            self._rng_mode, dense.KIND_NORMAL)
-
-    def _tf32_ok(self):
-        """Theta exact in TF32: float32 blocks can stay float32 (tcgen05 path, csrc/gemm32.cu)."""
-        return self._rng_mode in ("philox_rademacher", "philox_tf32")
-
-    def apply(self, U, mu=None):                                           # :425-434
-        torch = require_cuda()
-        V, kind = self._apply_sqrt_product(U)
-        if not (V.dtype == torch.float32 and self._tf32_ok() and not V.is_complex()):
-            V = V.to(torch.float64)
-        k = self.range.dim
-        result = torch.empty((V.shape[0], k), dtype=torch.float64, device=V.device)
-        # one plan (jump-ahead + acceptance count) for the streams of all blocks
-        plan = self._block_plan(V.device) if self._rng_mode == "mt19937" else None
-        off = 0
-        for i in range(len(self.block_sizes)):
-            b = self.block_sizes[i]
-            result[:, off:off + b].copy_(self._apply_block(i, V, plan))
-            off += b
-        return _wrap_result(kind, self.range, result)
-
-    def apply_adjoint(self, U, mu=None):
-        """V @ get_matrix()  (pyMOR's adjoint of the explicit matrix, embeddings.py:437-441), then Q^H.
-        On-the-fly modes: one kernel launch over all blocks with Theta generated in the kernel
-        (csrc/adjoint_rng.cu).  'mt19937': one plan for all blocks, each block drawn on the device in
-        turn and V[:, block] @ Theta_b accumulated, so one block of Theta is held at a time."""
-        k = self.range.dim
-        n = self.sqrt_product.range.dim
-        if self._rng_mode != "mt19937":
-            starts = np.concatenate([[0], np.cumsum(self.block_sizes)])
-            return self._gaussian_adjoint(
-                U, lambda v: dense.embed_adjoint_rng([int(s) for s in self.block_seeds], starts, self._kind(),
-                                                     1.0 / np.sqrt(k), v, n))
-
-        def product(v):
-            import torch
-            from .reductor_ops import gemm_nn
-            plan = self._block_plan(v.device)
-            out = torch.zeros((v.shape[0], n), dtype=torch.float64, device=v.device)
-            off = 0
-            for i, b in enumerate(self.block_sizes):
-                out += gemm_nn(v[:, off:off + b], self._draw_block_device(i, plan))
-                off += b
-            return out
-        return self._gaussian_adjoint(U, product)
-
-    def _block_plan(self, device):
-        n = self.sqrt_product.range.dim
-        return mt19937.NormalPlan(list(self.block_seeds), [b * n for b in self.block_sizes], device)
-
-    def _draw_block_device(self, i, plan):
-        """Row block i of Theta drawn on the device from a plan over all blocks."""
-        import torch
-        k = self.range.dim
-        n = self.sqrt_product.range.dim
-        b = self.block_sizes[i]
-        out = torch.empty((b, n), dtype=torch.float64, device=plan.device)
-        count = np.zeros(self.n_blocks, np.int64)
-        count[i] = b * n
-        if out.numel():
-            plan.execute(out.view(-1), 0, count, 0, 1 / np.sqrt(k))
-        return out
-
-    def _apply_block(self, i, V, plan=None):
-        """(m, b_i) sketch of the CUDA block V (already Q U) by row block i of Theta (:430-432)."""
-        k = self.range.dim
-        b = self.block_sizes[i]
-        if self._rng_mode == "mt19937":
-            # Theta blocks are not kept (the reference draws them again on every apply)
-            gauss = self._draw_block_device(i, plan if plan is not None else self._block_plan(V.device))
-            return dense.gauss_apply_explicit(gauss, V)
-        # independent stream per block: the block's own seed, rows 0..b-1
-        return dense.embed_apply_rng(int(self.block_seeds[i]), self._kind(), 1.0 / np.sqrt(k), b, V)
-
-    def _compute_matrix(self):                                             # :437-441
-        return self._adjoint_sqrt_product(self._compute_random_matrix())
-
-    def _compute_random_matrix(self):                                      # :444-450
-        if self._rng_mode == "mt19937" and _cuda_available():
-            k = self.range.dim
-            return mt19937.gaussian_matrix_host(list(self.block_seeds), self.block_sizes, self.sqrt_product.range.dim,
-                                                1 / np.sqrt(k))
-        return np.vstack([self._get_random_block(i) for i in range(self.n_blocks)])
+    @property
+    def _block_sizes(self):
+        return self.block_sizes
 
     def _get_random_block(self, ind):                                      # :452-461
-        k = self.range.dim
-        n = self.sqrt_product.range.dim
-        b = self.block_sizes[ind]
-        seed = self.block_seeds[ind]
-        if self._rng_mode == "mt19937":
-            if not _cuda_available():
-                return np.random.RandomState(seed).normal(size=(b, n), loc=0, scale=1 / np.sqrt(k))
-            return mt19937.gaussian_matrix([seed], [b], n, 1 / np.sqrt(k)).cpu().numpy()
-        return dense.theta_materialize(int(seed), self._kind(), 1.0 / np.sqrt(k), b, n).cpu().numpy()
+        return self._theta_host([ind])
 
     def get_block(self, ind):                                              # :463-467
         return self._adjoint_sqrt_product(self._get_random_block(ind))
 
-    def _get_random_block_device(self, ind):
-        require_cuda()
-        k = self.range.dim
-        n = self.sqrt_product.range.dim
-        if self._rng_mode == "mt19937":
-            return mt19937.gaussian_matrix([self.block_seeds[ind]], [self.block_sizes[ind]], n, 1 / np.sqrt(k))
-        return dense.theta_materialize(int(self.block_seeds[ind]), self._kind(), 1.0 / np.sqrt(k), self.block_sizes[ind], n)
-
     def get_block_device(self, ind):
         """Block `ind` of the U -> l2 matrix as a CUDA tensor (preconditioned_reductor.py:185-194)."""
-        return self._adjoint_sqrt_product_device(self._get_random_block_device(ind))
-
-    def _compute_random_matrix_device(self):
-        import torch
-        if self._rng_mode == "mt19937":
-            require_cuda()
-            return mt19937.gaussian_matrix(list(self.block_seeds), self.block_sizes, self.sqrt_product.range.dim,
-                                           1 / np.sqrt(self.range.dim))
-        return torch.cat([self._get_random_block_device(i) for i in range(self.n_blocks)], dim=0)
+        return self._adjoint_sqrt_product_device(self._theta_device([ind]))

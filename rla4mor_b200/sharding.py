@@ -94,30 +94,28 @@ def block_shard(n_blocks, rank, world):
     return list(range(lo, hi))
 
 
-def theta_row_sharded_sketch(local_sketch, k, rank, world, group=None, gather=True):
+def theta_row_sharded_sketch(local_sketch, k, rank, world, group=None, gather=True, ranges=None):
     """local_sketch(lo, hi) -> this rank's (m, hi - lo) columns of the sketch (rows lo..hi of Theta
-    applied to the replicated block).  No reduction is needed -- the slices are disjoint; with
-    `gather` they are concatenated along k on every rank by ONE all-gather, else the local slice
-    and its range are returned."""
+    applied to the replicated block).  `ranges` holds every rank's [lo, hi), `theta_row_shard` by
+    default.  No reduction is needed -- the slices are disjoint; with `gather` they are concatenated
+    along k on every rank by ONE all-gather, else the local slice and its range are returned."""
     import torch
     import torch.distributed as dist
-    lo, hi = theta_row_shard(k, rank, world)
+    if ranges is None:
+        ranges = [theta_row_shard(k, g, world) for g in range(world)]
+    lo, hi = ranges[rank]
     part = local_sketch(lo, hi)
     if not gather:
         return part, (lo, hi)
     if not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
         return part
     m = part.shape[0]
-    width = -(-int(k) // int(world))                  # slices differ by at most one column: pad to the widest
+    width = max(ghi - glo for glo, ghi in ranges)     # slices may differ in width: pad to the widest
     buf = torch.zeros((m, width), dtype=part.dtype, device=part.device)
     buf[:, :hi - lo] = part
     parts = [torch.empty_like(buf) for _ in range(world)]
     dist.all_gather(parts, buf, group=group)
-    cols = []
-    for g in range(world):
-        glo, ghi = theta_row_shard(k, g, world)
-        cols.append(parts[g][:, :ghi - glo])
-    return torch.cat(cols, dim=1)
+    return torch.cat([parts[g][:, :ghi - glo] for g, (glo, ghi) in enumerate(ranges)], dim=1)
 
 
 # --------------------------------------------------------------------- device front ends
@@ -138,30 +136,14 @@ def block_gaussian_theta_row_sharded(embedding, U, rank, world, group=None, gath
     the ranks: each rank regenerates only its own blocks (per-block seeds, :402-407) and the
     hstack of :433 becomes an all-gather.  U: replicated CUDA block (m, n)."""
     import torch
-    import torch.distributed as dist
     from .vectorarray import as_device_block
     V = as_device_block(U).to(torch.float64)
-    mine = block_shard(embedding.n_blocks, rank, world)
     offs = np.concatenate([[0], np.cumsum(embedding.block_sizes)])
-    cols = [embedding._apply_block(i, V) for i in mine]
-    part = torch.cat(cols, dim=1) if cols else torch.empty((V.shape[0], 0), dtype=torch.float64, device=V.device)
-    if not gather or not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
-        return part if gather else (part, (int(offs[mine[0]]) if mine else 0, int(offs[mine[-1] + 1]) if mine else 0))
-    k = int(offs[-1])
-    width = max(int(offs[block_shard(embedding.n_blocks, g, world)[-1] + 1] - offs[block_shard(embedding.n_blocks, g, world)[0]])
-                if block_shard(embedding.n_blocks, g, world) else 0 for g in range(world))
-    buf = torch.zeros((V.shape[0], width), dtype=torch.float64, device=V.device)
-    buf[:, :part.shape[1]] = part
-    parts = [torch.empty_like(buf) for _ in range(world)]
-    dist.all_gather(parts, buf, group=group)
-    out = []
-    for g in range(world):
-        bl = block_shard(embedding.n_blocks, g, world)
-        w = int(offs[bl[-1] + 1] - offs[bl[0]]) if bl else 0
-        out.append(parts[g][:, :w])
-    res = torch.cat(out, dim=1)
-    assert res.shape[1] == k
-    return res
+    shards = [block_shard(embedding.n_blocks, g, world) for g in range(world)]
+    ranges = [(int(offs[b[0]]), int(offs[b[-1] + 1])) if b else (0, 0) for b in shards]
+    return theta_row_sharded_sketch(lambda lo, hi: embedding.sketch_blocks(V, shards[rank]), int(offs[-1]), rank,
+                                    world, group, gather, ranges)
+
 
 def srht_row_sharded(x_slab, n, k, seed, rank, world, group=None, reducer=None, check=True):
     """Row-sharded SRHT on the GPU: x_slab is this rank's (m, hi - lo) CUDA slab.

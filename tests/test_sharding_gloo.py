@@ -59,18 +59,18 @@ def _worker(rank, world, port, n, k, seed, out):
         sl, rng = sharding.theta_row_sharded_sketch(lambda lo, hi: torch.from_numpy(x @ theta[lo:hi].T), k, rank, world,
                                                     gather=False)
         assert rng == sharding.theta_row_shard(k, rank, world) and sl.shape == (3, rng[1] - rng[0])
-        # blocks of a BlockGaussianEmbedding dealt to the ranks (embeddings.py:393-407)
+        # blocks of a BlockGaussianEmbedding dealt to the ranks (embeddings.py:393-407): uneven column
+        # ranges, an empty one with world 4
         sizes = eo.block_sizes(k, 7)
         seeds, _ = eo.block_seeds(seed, len(sizes))
-        mine = sharding.block_shard(len(sizes), rank, world)
-        cols = [x @ eo.block_gaussian_block(k, n, sizes[i], seeds[i]).T for i in mine]
-        width = max(sum(sizes[i] for i in sharding.block_shard(len(sizes), g, world)) for g in range(world))
-        buf = torch.zeros(3, width, dtype=torch.float64)
-        if cols:
-            c = np.hstack(cols); buf[:, :c.shape[1]] = torch.from_numpy(c)
-        parts = [torch.empty_like(buf) for _ in range(world)]
-        dist.all_gather(parts, buf)
-        yb = torch.cat([parts[g][:, :sum(sizes[i] for i in sharding.block_shard(len(sizes), g, world))] for g in range(world)], dim=1)
+        offs = np.concatenate([[0], np.cumsum(sizes)])
+        shards = [sharding.block_shard(len(sizes), g, world) for g in range(world)]
+        ranges = [(int(offs[b[0]]), int(offs[b[-1] + 1])) if b else (0, 0) for b in shards]
+
+        def local_blocks(lo, hi):
+            cols = [x @ eo.block_gaussian_block(k, n, sizes[i], seeds[i]).T for i in shards[rank]]
+            return torch.from_numpy(np.hstack(cols) if cols else np.zeros((3, 0)))
+        yb = sharding.theta_row_sharded_sketch(local_blocks, k, rank, world, ranges=ranges)
         if rank == 0:
             np.savez(out, y=y.numpy(), yg=yg.numpy(), yc=yc.numpy(), yt=yt.numpy(), yb=yb.numpy())
     finally:
