@@ -566,12 +566,17 @@ extern "C" int rla_sptrsv_solve_f64(const int64_t *rowptr_dev, const int32_t *co
     TrsvArgs a = {rowptr_dev, col_dev, val_dev, diag_eff_dev, split_dev, x_dev, ldx, m};
     const unsigned chunks = (unsigned)((ldx + TRSV_RHS - 1) / TRSV_RHS);
     RLA_REQUIRE(chunks <= 65535, "rla_sptrsv_solve_f64: too many right-hand sides");
-    static bool attr_set = false;
+    // the opt-in to 64 KB of dynamic shared memory holds for the current device only: made once per
+    // device, as a process may solve on several.  SparseLU.solve runs a shape eagerly before it
+    // captures it into a graph, so on its path the opt-in is never made during a capture.
+    static bool attr_set[64] = {};
+    int dev = 0;
+    RLA_CUDA_CHECK(cudaGetDevice(&dev));
     const int resolve_smem = TRSV_GROUP * 32 * (int)sizeof(double2);
-    if (!attr_set) {
+    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
         RLA_CUDA_CHECK(cudaFuncSetAttribute(trsv_resolve_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, resolve_smem));
         RLA_CUDA_CHECK(cudaFuncSetAttribute(trsv_resolve_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, resolve_smem));
-        attr_set = true;
+        if (dev >= 0 && dev < 64) attr_set[dev] = true;
     }
     for (int64_t s = 0; s < nsteps; ++s) {
         const int64_t cnt = step_hi[s] - step_lo[s];
