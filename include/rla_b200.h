@@ -401,6 +401,59 @@ int rla_residual_norm_batch_f64(const double *W_dev, int64_t ldw, int64_t Q, int
                                 const double *a_dev, int64_t lda, int64_t P, double *est_dev,
                                 void *ws_dev, size_t ws_bytes, void *stream);
 
+/* ------------------------------------- full-order solves over a parameter set ----
+ * Block preconditioned CG for the affine full-order model (csrc/affine_cg.cu): replaces, per mu_p,
+ * pyMOR's StationaryModel.solve -> apply_inverse of A(mu_p) = sum_q th[p, q] A_q (symmetric positive
+ * definite), with a host-factored SPD preconditioner R applied between the calls (the reductor's
+ * InverseLuOperator).  Every (P, n) block is row-major with row stride ld*; row p belongs to mu_p.
+ *
+ * rla_affine_spmm_f64:  y[p, :] = sum_q th[p, q] A_q x[p, :].  The operator is ONE CSR pattern
+ *   (rowptr n + 1 int64, col nnz int32), the union of the terms' patterns, with Q value arrays
+ *   val (Q, nnz) (0 where a term has no entry); th (P, Q; row stride ldth), 1 <= Q <= 32.  The
+ *   coefficient of an entry is formed per row p in ascending q with fma.  mode (int32 P, may be NULL)
+ *   restricts the product to the rows with mode[p] == 2; the other rows of y are not written.  With
+ *   ws != NULL the per-tile partial sums of <x_p, y_p> go to ws (see below).  Replaces the Q
+ *   MatrixOperator.apply calls and Q scaled additions of LincombOperator.apply.
+ * rla_row_dot_partials_f64:  per-tile partial sums of <a_p, b_p> (rows with mode[p] == 2, or all).
+ * rla_row_dot_sum_f64:  out[p] = the partials of row p added in tile order.
+ *   Workspace: rla_affine_cg_workspace_bytes(n, P) = 8 P ceil(n / 256) bytes, caller-owned; tile t of
+ *   row p (entries [256 t, 256 t + 256)) at ws[p ceil(n / 256) + t].  No atomics: the sums depend on
+ *   a row's own data only and are bit-identical from run to run.
+ *
+ * The CG state lives on the device: state (double, 5 x P) = rho, rho_b, alpha, beta, resid;
+ * istate (int32, 3 x P) = iterations, info, mode.  mode[p]: 2 = iterating, 1 = the row takes its
+ * last step in the coming update_xp, 0 = idle.  info[p]: 0 converged, 1 not converged within
+ * maxiter, 2 breakdown (<p, A p> <= 0 or <r, R^-1 r> < 0: A(mu) or R is not SPD; resid NaN).
+ * rla_affine_cg_start_f64:  from the partials of <r_0, R^-1 r_0> (ws_r) and <b, R^-1 b> (ws_b; the
+ *   same pointer when x_0 = 0) initialises every row: rho_b = 0 (b = 0) and rho_0 <= tol^2 rho_b
+ *   finish in 0 iterations, maxiter = 0 gives info 1, the rest iterate.
+ * rla_affine_cg_alpha_f64:  from the partials of <p, A p>: alpha = rho / <p, A p>, or breakdown.
+ * rla_affine_cg_update_r_f64:  r <- r - alpha A p on iterating rows.
+ * rla_affine_cg_beta_f64:  from the partials of <r, z> (z = R^-1 r): converged when
+ *   rho' <= tol^2 rho_b (||r||_{R^-1} <= tol ||b||_{R^-1}), out of iterations, breakdown, or
+ *   beta = rho' / rho; resid = sqrt(rho' / rho_b).  Rows that took their last step go idle.
+ * rla_affine_cg_update_xp_f64:  x <- x + alpha p on rows that took a step; p <- z + beta p on
+ *   rows that keep iterating. */
+size_t rla_affine_cg_workspace_bytes(int64_t n, int64_t P);
+int rla_affine_spmm_f64(const int64_t *rowptr_dev, const int32_t *col_dev, const double *val_dev, int64_t nnz, int64_t Q,
+                        int64_t n, const double *th_dev, int64_t ldth, const double *x_dev, int64_t ldx, int64_t P,
+                        double *y_dev, int64_t ldy, const int32_t *mode_dev, void *ws_dev, size_t ws_bytes,
+                        void *stream);
+int rla_row_dot_partials_f64(const double *a_dev, int64_t lda, const double *b_dev, int64_t ldb, int64_t n, int64_t P,
+                             const int32_t *mode_dev, void *ws_dev, size_t ws_bytes, void *stream);
+int rla_row_dot_sum_f64(const void *ws_dev, size_t ws_bytes, int64_t n, int64_t P, double *out_dev, void *stream);
+int rla_affine_cg_start_f64(const void *ws_r_dev, const void *ws_b_dev, size_t ws_bytes, int64_t n, int64_t P,
+                            double tol, int64_t maxiter, double *state_dev, int32_t *istate_dev, void *stream);
+int rla_affine_cg_alpha_f64(const void *ws_dev, size_t ws_bytes, int64_t n, int64_t P, double *state_dev,
+                            int32_t *istate_dev, void *stream);
+int rla_affine_cg_update_r_f64(double *r_dev, int64_t ldr, const double *q_dev, int64_t ldq, int64_t n, int64_t P,
+                               const double *state_dev, const int32_t *istate_dev, void *stream);
+int rla_affine_cg_beta_f64(const void *ws_dev, size_t ws_bytes, int64_t n, int64_t P, double tol, int64_t maxiter,
+                           double *state_dev, int32_t *istate_dev, void *stream);
+int rla_affine_cg_update_xp_f64(double *x_dev, int64_t ldx, double *p_dev, int64_t ldp, const double *z_dev,
+                                int64_t ldz, int64_t n, int64_t P, const double *state_dev, const int32_t *istate_dev,
+                                void *stream);
+
 /* --------------------------------------- sparse triangular solves (8f.1) ----
  * Device side of InverseLuOperator.apply / apply_adjoint (utilities/factorization.py:118-132,
  * `slu.solve(V.T).T`): the inverse_product R^-1 in front of the sketch

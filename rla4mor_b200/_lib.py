@@ -82,6 +82,16 @@ _SIGS = {
     "rla_residual_norm_batch_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "rla_residual_norm_batch_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, c_int64, _vp, c_int64, _vp,
                                             c_int64, _vp, c_int64, c_int64, _vp, _vp, c_size_t, _vp]),
+    "rla_affine_cg_workspace_bytes": (c_size_t, [c_int64, c_int64]),
+    "rla_affine_spmm_f64": (c_int, [_vp, _vp, _vp, c_int64, c_int64, c_int64, _vp, c_int64, _vp, c_int64, c_int64, _vp,
+                                    c_int64, _vp, _vp, c_size_t, _vp]),
+    "rla_row_dot_partials_f64": (c_int, [_vp, c_int64, _vp, c_int64, c_int64, c_int64, _vp, _vp, c_size_t, _vp]),
+    "rla_row_dot_sum_f64": (c_int, [_vp, c_size_t, c_int64, c_int64, _vp, _vp]),
+    "rla_affine_cg_start_f64": (c_int, [_vp, _vp, c_size_t, c_int64, c_int64, c_double, c_int64, _vp, _vp, _vp]),
+    "rla_affine_cg_alpha_f64": (c_int, [_vp, c_size_t, c_int64, c_int64, _vp, _vp, _vp]),
+    "rla_affine_cg_update_r_f64": (c_int, [_vp, c_int64, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp]),
+    "rla_affine_cg_beta_f64": (c_int, [_vp, c_size_t, c_int64, c_int64, c_double, c_int64, _vp, _vp, _vp]),
+    "rla_affine_cg_update_xp_f64": (c_int, [_vp, c_int64, _vp, c_int64, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp]),
     "rla_gram_schmidt_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "rla_gram_schmidt_status_offset": (c_int64, [c_int64, c_int64]),
     "rla_gram_schmidt_ws_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, _vp, _vp, c_double, c_double, c_double,

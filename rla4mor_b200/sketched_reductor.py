@@ -39,6 +39,24 @@ def _coef(c, mu):
     return float(c)
 
 
+def _theta_rows(fom, theta_lhs, theta_rhs, mus, Q, Pf, dev):
+    """theta_lhs (P, Q) and theta_rhs (P, Pf) as given (the fast path), or fom.thetas of every
+    entry of `mus` stacked on the host and uploaded once; ValueError on a missing argument or a
+    shape mismatch."""
+    if mus is not None:
+        if theta_lhs is not None or theta_rhs is not None:
+            raise ValueError("give either mus= or theta_lhs= / theta_rhs=, not both")
+        theta_lhs, theta_rhs = fom.thetas_batch(mus)
+    elif theta_lhs is None or theta_rhs is None:
+        raise ValueError("give mus= or both theta_lhs= and theta_rhs=")
+    th = torch.as_tensor(theta_lhs, dtype=torch.float64, device=dev)
+    tf = torch.as_tensor(theta_rhs, dtype=torch.float64, device=dev)
+    if th.dim() != 2 or th.shape[1] != Q or tf.dim() != 2 or tf.shape != (th.shape[0], Pf):
+        raise ValueError(f"theta_lhs / theta_rhs: expected shapes (P, {Q}) and (P, {Pf}), "
+                         f"got {tuple(th.shape)} and {tuple(tf.shape)}")
+    return th, tf
+
+
 class AffineModel:
     """Stationary affine full-order model  sum_q thA_q(mu) A_q u = sum_p thf_p(mu) f_p,
     output L u.  operators: objects with `.apply(DeviceVectorArray)` (e.g. MatrixOperator);
@@ -55,6 +73,7 @@ class AffineModel:
         if solution_space is None:
             solution_space = getattr(self.operators[0], "source", None) or DeviceVectorSpace(self.rhs[0].shape[1])
         self.solution_space = solution_space
+        self._affine = None                      # the terms as one device CSR pattern, built by the first solve
 
     def thetas(self, mu):
         return ([_coef(c, mu) for c in self.operator_coefficients], [_coef(c, mu) for c in self.rhs_coefficients])
@@ -66,6 +85,38 @@ class AffineModel:
         for p, mu in enumerate(mus):
             th[p], tf[p] = self.thetas(mu)
         return th, tf
+
+    def solve(self, mu=None, theta_lhs=None, theta_rhs=None, *, preconditioner, tol=1e-10, maxiter=500, x0=None,
+              check=True):
+        """The full-order solution u(mu) (pyMOR's StationaryModel.solve) as a DeviceVectorArray of
+        length 1 in solution_space: solve_batch of one mu (`mu=`, or theta_lhs (Q,) and theta_rhs
+        (Pf,)); x0 is an optional initial guess of length 1."""
+        one = lambda t: None if t is None else torch.as_tensor(t, dtype=torch.float64)[None]
+        return self.solve_batch(None if mu is None else [mu], one(theta_lhs), one(theta_rhs),
+                                preconditioner=preconditioner, tol=tol, maxiter=maxiter, x0=x0, check=check)
+
+    def solve_batch(self, mus=None, theta_lhs=None, theta_rhs=None, *, preconditioner, tol=1e-10, maxiter=500,
+                    x0=None, check=True):
+        """Full-order solutions u(mu_p) of every mu, a DeviceVectorArray of length P in
+        solution_space, by block preconditioned CG on the device (fom_solve.affine_cg: one affine
+        SpMM, one application of `preconditioner` to the whole block and a few vector kernels per
+        iteration).  The parameters are `mus=` or theta_lhs (P, Q) and theta_rhs (P, Pf), as for
+        SketchedRom.solve_batch.  Every term must be a symmetric sparse MatrixOperator and A(mu) SPD;
+        `preconditioner` is an SPD operator such as the reductor's `inverse_product`.  Row p stops when
+        ||r_p||_{R^-1} <= tol ||b_p||_{R^-1}.  A row that does not converge within `maxiter`
+        iterations or breaks down raises RlaError; with check=False it is returned as is (its last
+        iterate, or NaN after a breakdown)."""
+        from . import fom_solve
+        dev = self.rhs[0].device if self.rhs else torch.device("cuda", torch.cuda.current_device())
+        th, tf = _theta_rows(self, theta_lhs, theta_rhs, mus, len(self.operators), len(self.rhs), dev)
+        n = self.solution_space.dim
+        if x0 is not None:
+            x0 = fom_solve.check_block(x0, th.shape[0], n, "x0", dev)
+        if self._affine is None:
+            self._affine = fom_solve.AffineCsr(self.operators)               # once per model
+        X = fom_solve.affine_cg(self._affine, self.rhs, th, tf, preconditioner, tol=tol, maxiter=maxiter, x0=x0,
+                                check=check)[0]
+        return DeviceVectorArray(self.solution_space, X)
 
 
 class SketchedReductor:
@@ -280,22 +331,8 @@ class SketchedRom:
         return self.est_lhs_rows[0].shape[0]                    # (r, k') for both projections
 
     def _thetas_batch(self, theta_lhs, theta_rhs, mus):
-        """theta_lhs (P, Q) and theta_rhs (P, Pf) as given (the fast path), or fom.thetas of every
-        entry of `mus` stacked on the host and uploaded once."""
-        if mus is not None:
-            if theta_lhs is not None or theta_rhs is not None:
-                raise ValueError("give either mus= or theta_lhs= / theta_rhs=, not both")
-            theta_lhs, theta_rhs = self.fom.thetas_batch(mus)
-        elif theta_lhs is None or theta_rhs is None:
-            raise ValueError("give mus= or both theta_lhs= and theta_rhs=")
-        dev = self.output_functional.device
-        th = torch.as_tensor(theta_lhs, dtype=torch.float64, device=dev)
-        tf = torch.as_tensor(theta_rhs, dtype=torch.float64, device=dev)
-        Q, Pf = len(self.est_lhs_rows), len(self.est_rhs)
-        if th.dim() != 2 or th.shape[1] != Q or tf.dim() != 2 or tf.shape != (th.shape[0], Pf):
-            raise ValueError(f"theta_lhs / theta_rhs: expected shapes (P, {Q}) and (P, {Pf}), "
-                             f"got {tuple(th.shape)} and {tuple(tf.shape)}")
-        return th, tf
+        return _theta_rows(self.fom, theta_lhs, theta_rhs, mus, len(self.est_lhs_rows), len(self.est_rhs),
+                           self.output_functional.device)
 
     def _batch_a(self, a, th, tf):
         if a is None:
