@@ -27,26 +27,14 @@ import pytest
 import scipy.sparse as sp
 from scipy.sparse.linalg import splu
 
+from exact_ref import U_ROUND, gamma, require_longdouble, two_product
 from rla4mor_b200.factorization import plan_triangular, splu_symetric
 from test_sptrsv_plan import _replay
 
 pytestmark = pytest.mark.gpu
 
-U_ROUND = 2.0 ** -53                                   # unit roundoff of float64
-
-
-def gamma(k):
-    """gamma_k = k u / (1 - k u) (Higham, Accuracy and Stability, section 3.1)."""
-    k = np.asarray(k, dtype=np.float64)
-    return k * U_ROUND / (1.0 - k * U_ROUND)
-
 
 # ---------------------------------------------------------------- extended-precision reference
-
-def require_longdouble():
-    if np.finfo(np.longdouble).nmant < 63:
-        pytest.skip("np.longdouble is not the 64-bit-mantissa extended format on this platform")
-
 
 def substitute(T, B, lower):
     """T X = B by substitution over the CSR rows of T in np.longdouble (64-bit mantissa), all
@@ -83,23 +71,6 @@ def exact_lu_solve(factorization, B, adjoint=False):
     else:
         Z = substitute(U, substitute(L, Y, True), False)
     return Z[p_out].T
-
-
-_SPLIT = 134217729.0                                   # 2^27 + 1
-
-
-def two_product(a, b):
-    """a * b = p + e exactly (Dekker's TwoProduct with Veltkamp's split; float64 arithmetic,
-    no fused multiply-add).  Exact while no product or split part under- or overflows."""
-    p = a * b
-    c = _SPLIT * a
-    ah = c - (c - a)
-    al = a - ah
-    c = _SPLIT * b
-    bh = c - (c - b)
-    bl = b - bh
-    e = ((ah * bh - p) + ah * bl + al * bh) + al * bl
-    return p, e
 
 
 def exact_residual(T, X, B):
