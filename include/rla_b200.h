@@ -454,6 +454,58 @@ int rla_affine_cg_update_xp_f64(double *x_dev, int64_t ldx, double *p_dev, int64
                                 int64_t ldz, int64_t n, int64_t P, const double *state_dev, const int32_t *istate_dev,
                                 void *stream);
 
+/* Restarted GMRES(m) for the affine full-order model (csrc/affine_gmres.cu): A(mu_p) need be neither
+ * symmetric nor definite.  Left preconditioning by R^-1 (SPD, applied between the calls) with the
+ * basis orthogonal in the R inner product: row p minimises ||b_p - A x_p||_{R^-1}.  Each row keeps
+ * V (primal basis) and W = R V (dual basis), both (P, m, n) with row p's m vectors contiguous, so
+ * <z, v_i>_R = <z, w_i>.  Blocks z = R^-1 y, y, U, x, b are (P, n) contiguous.
+ *
+ * istate (int32, 10 x P): iterations (Arnoldi steps), info, mode (0 idle, 1 in a cycle, 2 restart),
+ * ncol (basis vectors of the cycle), cycles, then the masks (2 = yes, 0 = no) act (the row takes
+ * part in this step's affine SpMM: y = A U), arn (an Arnoldi step), reorth (a second Gram-Schmidt
+ * pass), restart (y = b - A x, the true residual) and end (the cycle ended: x += V y).
+ * state (double, 5 x P): <b, R^-1 b>, resid, the next normalisation 1/h, ||z||_R^2 before and after
+ * the first pass.  hess (rla_affine_gmres_hess_bytes): per row H (m + 1, m) row-major, g (m + 1),
+ * the rotations' cosines (m) and sines (m), and the triangle's solution (m).
+ * info: 0 converged (the true residual at a cycle start within tol), 1 out of iterations (last
+ * iterate), 2 breakdown (<r, R^-1 r> < 0, <z, y> < 0, a singular triangle or a non-finite value).
+ *
+ * One Arnoldi step: rla_affine_spmm_f64 (U -> y, mask act); rla_affine_gmres_residual_f64; z = R^-1 y;
+ * rla_affine_gmres_dots_f64 (mask act) + rla_row_dot_sum_f64 over P (m + 2) rows -> hb (P, m + 2);
+ * rla_affine_gmres_orth_f64 (mask arn) + rla_row_dot_sum_f64 -> hb2 (P); rla_affine_gmres_dgks_f64;
+ * dots, sums and orth again with mask reorth; rla_affine_gmres_step_f64;
+ * rla_affine_gmres_normalize_f64; rla_affine_gmres_update_f64.
+ * rla_affine_gmres_dots_f64:  per-tile partials of <z_p, w_{p,k}> (k < c) and <z_p, y_p> (k = c) at
+ *   ws[(p (m + 2) + k) ceil(n / 256) + tile], c = ncol in a cycle and 0 at a restart.  Workspace
+ *   rla_affine_gmres_workspace_bytes(n, m, P) = 8 P (m + 2) ceil(n / 256).
+ * rla_affine_gmres_orth_f64:  z -= sum_{k<c} hb[p, k] v_k, y -= sum_{k<c} hb[p, k] w_k, and the
+ *   per-tile partials of <z', y'> (workspace 8 P ceil(n / 256) bytes).
+ * rla_affine_gmres_dgks_f64:  column c - 1 of H from hb; reorth when ||z'||_R^2 < ||z||_R^2 / 2.
+ * rla_affine_gmres_step_f64:  a restart row: converged, out of iterations, breakdown or a new cycle
+ *   (g = beta e_0); an Arnoldi row: h_{c,c-1} = ||z'||_R, Givens rotations, and the end of the cycle
+ *   (c = m, |g_c| <= tol ||b||_{R^-1}, h = 0 or maxiter) with the triangle solved.
+ * rla_affine_gmres_normalize_f64:  v_{c-1} = z' s, w_{c-1} = y' s, U = v_{c-1} (mask arn).
+ * rla_affine_gmres_update_f64:  x += sum_{k<c} y_k v_k and U = x (mask end). */
+size_t rla_affine_gmres_workspace_bytes(int64_t n, int64_t m, int64_t P);
+size_t rla_affine_gmres_hess_bytes(int64_t m, int64_t P);
+int rla_affine_gmres_dots_f64(const double *z_dev, const double *y_dev, const double *W_dev, int64_t n, int64_t m,
+                              int64_t P, const int32_t *istate_dev, const int32_t *mask_dev, void *ws_dev,
+                              size_t ws_bytes, void *stream);
+int rla_affine_gmres_orth_f64(double *z_dev, double *y_dev, const double *V_dev, const double *W_dev,
+                              const double *hb_dev, int64_t n, int64_t m, int64_t P, const int32_t *istate_dev,
+                              const int32_t *mask_dev, void *ws_dev, size_t ws_bytes, void *stream);
+int rla_affine_gmres_dgks_f64(const double *hb_dev, const double *hb2_dev, int64_t m, int64_t P, double *state_dev,
+                              int32_t *istate_dev, double *hess_dev, void *stream);
+int rla_affine_gmres_step_f64(const double *hb_dev, const double *hb2_dev, int64_t m, int64_t P, double tol,
+                              int64_t maxiter, double *state_dev, int32_t *istate_dev, double *hess_dev, void *stream);
+int rla_affine_gmres_residual_f64(double *y_dev, const double *b_dev, int64_t n, int64_t P, const int32_t *istate_dev,
+                                  void *stream);
+int rla_affine_gmres_normalize_f64(const double *z_dev, const double *y_dev, double *V_dev, double *W_dev,
+                                   double *U_dev, int64_t n, int64_t m, int64_t P, const double *state_dev,
+                                   const int32_t *istate_dev, void *stream);
+int rla_affine_gmres_update_f64(double *x_dev, double *U_dev, const double *V_dev, int64_t n, int64_t m, int64_t P,
+                                const int32_t *istate_dev, const double *hess_dev, void *stream);
+
 /* --------------------------------------- sparse triangular solves (8f.1) ----
  * Device side of InverseLuOperator.apply / apply_adjoint (utilities/factorization.py:118-132,
  * `slu.solve(V.T).T`): the inverse_product R^-1 in front of the sketch

@@ -92,6 +92,16 @@ _SIGS = {
     "rla_affine_cg_update_r_f64": (c_int, [_vp, c_int64, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp]),
     "rla_affine_cg_beta_f64": (c_int, [_vp, c_size_t, c_int64, c_int64, c_double, c_int64, _vp, _vp, _vp]),
     "rla_affine_cg_update_xp_f64": (c_int, [_vp, c_int64, _vp, c_int64, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp]),
+    "rla_affine_gmres_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
+    "rla_affine_gmres_hess_bytes": (c_size_t, [c_int64, c_int64]),
+    "rla_affine_gmres_dots_f64": (c_int, [_vp, _vp, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp, c_size_t, _vp]),
+    "rla_affine_gmres_orth_f64": (c_int, [_vp, _vp, _vp, _vp, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp, c_size_t,
+                                          _vp]),
+    "rla_affine_gmres_dgks_f64": (c_int, [_vp, _vp, c_int64, c_int64, _vp, _vp, _vp, _vp]),
+    "rla_affine_gmres_step_f64": (c_int, [_vp, _vp, c_int64, c_int64, c_double, c_int64, _vp, _vp, _vp, _vp]),
+    "rla_affine_gmres_residual_f64": (c_int, [_vp, _vp, c_int64, c_int64, _vp, _vp]),
+    "rla_affine_gmres_normalize_f64": (c_int, [_vp, _vp, _vp, _vp, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp]),
+    "rla_affine_gmres_update_f64": (c_int, [_vp, _vp, _vp, c_int64, c_int64, c_int64, _vp, _vp, _vp]),
     "rla_gram_schmidt_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "rla_gram_schmidt_status_offset": (c_int64, [c_int64, c_int64]),
     "rla_gram_schmidt_ws_f64": (c_int, [_vp, c_int64, c_int64, c_int64, c_int64, _vp, _vp, c_double, c_double, c_double,

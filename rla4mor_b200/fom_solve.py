@@ -75,7 +75,8 @@ def union_pattern(matrices):
 class AffineCsr:
     """sum_q th_q A_q of sparse `MatrixOperator`s as one device CSR pattern (the union of the terms'
     patterns) with Q value arrays: the operator the affine SpMM of csrc/affine_cg.cu applies with
-    one coefficient vector per row of the block.  Built once per model."""
+    one coefficient vector per row of the block.  Built once per model.  `symmetric` records whether
+    every term is symmetric (to SYMMETRY_RTOL): affine_cg needs it, affine_gmres does not."""
 
     def __init__(self, operators):
         operators = list(operators)
@@ -87,7 +88,16 @@ class AffineCsr:
         if len(operators) > MAX_TERMS:
             raise ValueError(f"AffineCsr: {len(operators)} affine terms, at most {MAX_TERMS} supported")
         mats = [A._host for A in operators]
-        check_symmetric(mats)
+        for q, M in enumerate(mats):
+            if M.shape[0] != M.shape[1]:
+                raise ValueError(f"affine term {q} is not square: shape {M.shape}")
+        # GMRES takes any terms, CG symmetric ones only: the first asymmetry is kept for affine_cg's error
+        try:
+            check_symmetric(mats)
+            self.asymmetry = None
+        except ValueError as e:
+            self.asymmetry = str(e)
+        self.symmetric = self.asymmetry is None
         indptr, indices, values = union_pattern(mats)
         self.source = operators[0].source
         self.n, self.Q, self.nnz = int(mats[0].shape[0]), len(mats), int(indices.size)
@@ -159,6 +169,8 @@ def affine_cg(operators, rhs, th, tf, preconditioner, tol=1e-10, maxiter=500, x0
     <r, R^-1 r> < 0: A(mu) or the preconditioner is not SPD; the row is NaN).  With `check`, a
     nonzero info raises RlaError naming how many rows failed, the first one and why."""
     A = operators if isinstance(operators, AffineCsr) else AffineCsr(operators)
+    if not A.symmetric:
+        raise ValueError(A.asymmetry)
     n, Q, dev = A.n, A.Q, A.device
     th = torch.as_tensor(th)
     P = int(th.shape[0]) if th.dim() == 2 else -1
@@ -250,3 +262,188 @@ def affine_cg(operators, rhs, th, tf, preconditioner, tol=1e-10, maxiter=500, x0
                            + (f", relative residual {res:.3g} after {maxiter} iterations)" if why == 1 else ")"))
     return X, iters, resid, info
 
+
+
+# ---------------------------------------------------------------------------- GMRES
+# The Krylov storage of affine_gmres, 2 m + 5 blocks (P, n), stays within this share of the free
+# device memory (the rule of SketchedReductor.extend_basis); a larger P runs in chunks of rows.
+KRYLOV_MEMORY_FRACTION = 0.25
+# istate rows of csrc/affine_gmres.cu
+_G_ITERS, _G_INFO, _G_MODE, _G_NCOL, _G_CYCLES, _G_ACT, _G_ARN, _G_REORTH, _G_RESTART, _G_END = range(10)
+_G_MODE_RESTART = 2
+_INFO_GMRES = {1: "not converged within maxiter",
+               2: "breakdown: the preconditioner is not SPD or A(mu) is singular"}
+
+
+def _check_restart(restart, who):
+    if isinstance(restart, bool) or not isinstance(restart, (int, np.integer)) or restart < 1:
+        raise ValueError(f"{who}: restart={restart!r} must be an integer >= 1")
+    return int(restart)
+
+
+def gmres_rows_per_chunk(n, m, P, free_bytes):
+    """Rows of the block solved at once: the 2 m + 5 blocks of length n per row (V, W, x, b, U, y,
+    z) and the reductions' workspace within KRYLOV_MEMORY_FRACTION of `free_bytes`; at least 1."""
+    per_row = (2 * m + 5) * n * 8 + (m + 3) * ((n + 255) // 256) * 8
+    return max(1, min(P, int(KRYLOV_MEMORY_FRACTION * free_bytes) // per_row))
+
+
+def affine_gmres(operators, rhs, th, tf, preconditioner, tol=1e-10, restart=30, maxiter=500, x0=None, check=True):
+    """Restarted GMRES(m) for  (sum_q th[p, q] A_q) x_p = sum_j tf[p, j] f_j,  p = 0 .. P-1, where
+    A(mu) may be non-symmetric or indefinite (csrc/affine_gmres.cu).
+
+    The arguments are those of affine_cg, plus `restart` = m, the Arnoldi steps of a cycle.  The
+    iteration is GMRES on R^-1 A(mu) (left preconditioning by the SPD `preconditioner`) with the
+    basis orthogonal in the R inner product, so that row p minimises ||b_p - A x_p||_{R^-1} over its
+    Krylov space; a second Gram-Schmidt pass is taken when the first one loses more than half of
+    the vector's R-norm (DGKS).  A cycle ends after m steps or when the Givens estimate of the
+    residual reaches tol; the row converges only when the residual recomputed at the next cycle
+    start satisfies ||r_p||_{R^-1} <= tol ||b_p||_{R^-1}.
+
+    Returns (X (P, n), iters (P,) int32 -- Arnoldi steps, resid (P,) -- the true relative residual
+    at the last cycle start, info (P,) int32) on the device: info 0 converged, 1 not converged
+    within `maxiter` steps (the row keeps its last iterate), 2 breakdown (<r, R^-1 r> < 0 or
+    <z, R z> < 0: the preconditioner is not SPD; a singular A(mu); a non-finite value; the row is
+    NaN).  A row with b_p = 0 is 0 after 0 steps.  Rows are independent; the Krylov storage,
+    2 m + 5 blocks of (rows, n), is kept within KRYLOV_MEMORY_FRACTION of the free device memory
+    by solving the rows in chunks.  With `check`, a nonzero info raises RlaError."""
+    X, iters, resid, info, _ = _affine_gmres(operators, rhs, th, tf, preconditioner, tol, restart, maxiter, x0)
+    if check:
+        _raise_failed("affine_gmres", _INFO_GMRES, info, resid, maxiter)
+    return X, iters, resid, info
+
+
+def _raise_failed(who, reasons, info, resid, maxiter):
+    P = info.numel()
+    bad = info != 0
+    first = torch.argmax(bad.to(torch.int32))
+    n_bad, first, why, res = torch.stack([bad.sum().to(torch.float64), first.to(torch.float64),
+                                          info[first].to(torch.float64), resid[first]]).tolist()
+    if n_bad:
+        raise RlaError(f"{who}: {int(n_bad)} of {P} rows failed (first: row {int(first)}, {reasons[int(why)]}"
+                       + (f", relative residual {res:.3g} after {maxiter} iterations)" if why == 1 else ")"))
+
+
+def _affine_gmres(operators, rhs, th, tf, preconditioner, tol, restart, maxiter, x0):
+    """affine_gmres without the check: (X, iters, resid, info, cycles)."""
+    m = _check_restart(restart, "affine_gmres")
+    if not tol >= 0.0:
+        raise ValueError(f"affine_gmres: tol={tol} must be >= 0")
+    if isinstance(maxiter, bool) or int(maxiter) != maxiter or maxiter < 0:
+        raise ValueError(f"affine_gmres: maxiter={maxiter} must be a non-negative integer")
+    maxiter = int(maxiter)
+    A = operators if isinstance(operators, AffineCsr) else AffineCsr(operators)
+    n, Q, dev = A.n, A.Q, A.device
+    th = torch.as_tensor(th)
+    P = int(th.shape[0]) if th.dim() == 2 else -1
+    if isinstance(rhs, torch.Tensor):
+        F = rhs.to(device=dev, dtype=torch.float64).reshape(-1, n)
+    else:
+        F = torch.cat([as_device_block(f).to(torch.float64).reshape(-1, n) for f in rhs] +
+                      [torch.empty((0, n), dtype=torch.float64, device=dev)], dim=0)
+    Pf = int(F.shape[0])
+    th, ldth = ops._param_rows(th, P, Q, "affine_gmres: th", dev)
+    tf, _ = ops._param_rows(tf, P, Pf, "affine_gmres: tf", dev)
+    if x0 is not None:
+        x0 = check_block(x0, P, n, "affine_gmres: x0", dev)
+    m = max(1, min(m, maxiter))             # a cycle never outlasts maxiter: the same iterates, less storage
+    iters = torch.zeros((P,), dtype=torch.int32, device=dev)
+    info = torch.zeros((P,), dtype=torch.int32, device=dev)
+    cycles = torch.zeros((P,), dtype=torch.int32, device=dev)
+    resid = torch.zeros((P,), dtype=torch.float64, device=dev)
+    X = torch.empty((P, n), dtype=torch.float64, device=dev)
+    if P == 0:
+        return X, iters, resid, info, cycles
+    space = getattr(preconditioner, "source", A.source)
+
+    def precond(V):
+        Z = preconditioner.apply(DeviceVectorArray(space, V)).data
+        if tuple(Z.shape) != tuple(V.shape):
+            raise ValueError(f"affine_gmres: the preconditioner returned shape {tuple(Z.shape)} for {tuple(V.shape)}")
+        return Z.to(torch.float64).contiguous()
+
+    tf = tf.contiguous()
+    with torch.cuda.device(dev):
+        chunk = gmres_rows_per_chunk(n, m, P, torch.cuda.mem_get_info(dev)[0])
+        for p0 in range(0, P, chunk):
+            p1 = min(P, p0 + chunk)
+            B = ops.gemm_nn(tf[p0:p1], F) if Pf else torch.zeros((p1 - p0, n), dtype=torch.float64, device=dev)
+            out = _gmres_block(A, th[p0:], ldth, B, None if x0 is None else x0[p0:p1], precond, float(tol), m, maxiter)
+            for dst, src in zip((X, iters, resid, info, cycles), out):
+                dst[p0:p1] = src
+    return X, iters, resid, info, cycles
+
+
+def _gmres_block(A, th, ldth, B, X, precond, tol, m, maxiter):
+    """GMRES(m) on the rows of B (P, n) with coefficients th (row stride ldth); X: the initial
+    guess (modified in place) or None.  (X, iters, resid, info, cycles)."""
+    L, s = lib(), stream_ptr
+    P, n = B.shape
+    dev = B.device
+    f64 = dict(dtype=torch.float64, device=dev)
+    ist = torch.zeros((10, P), dtype=torch.int32, device=dev)
+    st = torch.zeros((5, P), **f64)                       # <b, R^-1 b>, resid, 1/h, ||z||_R^2 before / after
+    hess = torch.zeros((L.rla_affine_gmres_hess_bytes(m, P) // 8,), **f64)
+    V = torch.empty((P, m, n), **f64)
+    W = torch.empty((P, m, n), **f64)
+    U = torch.empty((P, n), **f64)
+    ws = dense._workspace(L.rla_affine_gmres_workspace_bytes(n, m, P), dev)
+    ws2 = dense._workspace(L.rla_affine_cg_workspace_bytes(n, P), dev)
+    hb = torch.empty((P, m + 2), **f64)
+    hb2 = torch.empty((P,), **f64)
+    act, arn, reorth, rst = ist[_G_ACT], ist[_G_ARN], ist[_G_REORTH], ist[_G_RESTART]
+    ist[_G_MODE].fill_(_G_MODE_RESTART)                  # every row starts with its true residual
+    act.fill_(_LIVE)
+    rst.fill_(_LIVE)
+    if X is None:
+        X = torch.zeros((P, n), **f64)
+        Y = B.clone()                                     # r_0 = b
+        Z = precond(Y)
+        Zb = Z
+    else:
+        Y = torch.empty_like(X)
+        _spmm(A, th, ldth, X, Y, act, None)
+        _lib.check(L.rla_affine_gmres_residual_f64(Y.data_ptr(), B.data_ptr(), n, P, ist.data_ptr(), s()),
+                   "rla_affine_gmres_residual_f64")
+        ZZ = precond(torch.cat([Y, B], dim=0))            # R^-1 of r_0 and of b in one solve
+        Z, Zb = ZZ[:P], ZZ[P:]
+    _dots(B, Zb, n, None, ws2)
+    _lib.check(L.rla_row_dot_sum_f64(ws2.data_ptr(), ws2.numel(), n, P, st[0].data_ptr(), s()), "rla_row_dot_sum_f64")
+
+    def gram_schmidt_pass(mask_dots, mask_orth):
+        _lib.check(L.rla_affine_gmres_dots_f64(Z.data_ptr(), Y.data_ptr(), W.data_ptr(), n, m, P, ist.data_ptr(),
+                                               mask_dots.data_ptr(), ws.data_ptr(), ws.numel(), s()),
+                   "rla_affine_gmres_dots_f64")
+        _lib.check(L.rla_row_dot_sum_f64(ws.data_ptr(), ws.numel(), n, P * (m + 2), hb.data_ptr(), s()),
+                   "rla_row_dot_sum_f64")
+        _lib.check(L.rla_affine_gmres_orth_f64(Z.data_ptr(), Y.data_ptr(), V.data_ptr(), W.data_ptr(), hb.data_ptr(),
+                                               n, m, P, ist.data_ptr(), mask_orth.data_ptr(), ws2.data_ptr(),
+                                               ws2.numel(), s()), "rla_affine_gmres_orth_f64")
+        _lib.check(L.rla_row_dot_sum_f64(ws2.data_ptr(), ws2.numel(), n, P, hb2.data_ptr(), s()),
+                   "rla_row_dot_sum_f64")
+
+    first = True
+    while True:
+        if not first:
+            _spmm(A, th, ldth, U, Y, act, None)           # A v_j, or A x at a restart
+            _lib.check(L.rla_affine_gmres_residual_f64(Y.data_ptr(), B.data_ptr(), n, P, ist.data_ptr(), s()),
+                       "rla_affine_gmres_residual_f64")
+            Z = precond(Y)
+        first = False
+        gram_schmidt_pass(act, arn)
+        _lib.check(L.rla_affine_gmres_dgks_f64(hb.data_ptr(), hb2.data_ptr(), m, P, st.data_ptr(), ist.data_ptr(),
+                                               hess.data_ptr(), s()), "rla_affine_gmres_dgks_f64")
+        gram_schmidt_pass(reorth, reorth)
+        _lib.check(L.rla_affine_gmres_step_f64(hb.data_ptr(), hb2.data_ptr(), m, P, tol, maxiter, st.data_ptr(),
+                                               ist.data_ptr(), hess.data_ptr(), s()), "rla_affine_gmres_step_f64")
+        _lib.check(L.rla_affine_gmres_normalize_f64(Z.data_ptr(), Y.data_ptr(), V.data_ptr(), W.data_ptr(),
+                                                    U.data_ptr(), n, m, P, st.data_ptr(), ist.data_ptr(), s()),
+                   "rla_affine_gmres_normalize_f64")
+        _lib.check(L.rla_affine_gmres_update_f64(X.data_ptr(), U.data_ptr(), V.data_ptr(), n, m, P, ist.data_ptr(),
+                                                 hess.data_ptr(), s()), "rla_affine_gmres_update_f64")
+        if not bool((act == _LIVE).any()):                # the one device-to-host read per step
+            break
+    info = ist[_G_INFO].clone()
+    X[info == 2] = float("nan")
+    X[st[0] == 0] = 0.0                                   # b_p = 0: x_p = 0
+    return X, ist[_G_ITERS].clone(), st[1].clone(), info, ist[_G_CYCLES].clone()

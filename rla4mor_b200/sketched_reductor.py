@@ -87,26 +87,44 @@ class AffineModel:
         return th, tf
 
     def solve(self, mu=None, theta_lhs=None, theta_rhs=None, *, preconditioner, tol=1e-10, maxiter=500, x0=None,
-              check=True):
+              check=True, method='cg', restart=None):
         """The full-order solution u(mu) (pyMOR's StationaryModel.solve) as a DeviceVectorArray of
         length 1 in solution_space: solve_batch of one mu (`mu=`, or theta_lhs (Q,) and theta_rhs
         (Pf,)); x0 is an optional initial guess of length 1."""
         one = lambda t: None if t is None else torch.as_tensor(t, dtype=torch.float64)[None]
         return self.solve_batch(None if mu is None else [mu], one(theta_lhs), one(theta_rhs),
-                                preconditioner=preconditioner, tol=tol, maxiter=maxiter, x0=x0, check=check)
+                                preconditioner=preconditioner, tol=tol, maxiter=maxiter, x0=x0, check=check,
+                                method=method, restart=restart)
 
     def solve_batch(self, mus=None, theta_lhs=None, theta_rhs=None, *, preconditioner, tol=1e-10, maxiter=500,
-                    x0=None, check=True):
+                    x0=None, check=True, method='cg', restart=None):
         """Full-order solutions u(mu_p) of every mu, a DeviceVectorArray of length P in
-        solution_space, by block preconditioned CG on the device (fom_solve.affine_cg: one affine
-        SpMM, one application of `preconditioner` to the whole block and a few vector kernels per
-        iteration).  The parameters are `mus=` or theta_lhs (P, Q) and theta_rhs (P, Pf), as for
-        SketchedRom.solve_batch.  Every term must be a symmetric sparse MatrixOperator and A(mu) SPD;
-        `preconditioner` is an SPD operator such as the reductor's `inverse_product`.  Row p stops when
-        ||r_p||_{R^-1} <= tol ||b_p||_{R^-1}.  A row that does not converge within `maxiter`
-        iterations or breaks down raises RlaError; with check=False it is returned as is (its last
-        iterate, or NaN after a breakdown)."""
+        solution_space, by a block Krylov method on the device: one affine SpMM, one application of
+        `preconditioner` to the whole block and a few vector kernels per iteration.  The parameters
+        are `mus=` or theta_lhs (P, Q) and theta_rhs (P, Pf), as for SketchedRom.solve_batch.
+        `preconditioner` is an SPD operator R such as the reductor's `inverse_product`; row p stops
+        when ||r_p||_{R^-1} <= tol ||b_p||_{R^-1}.
+
+        method='cg' (default): block preconditioned CG (fom_solve.affine_cg).  Every term must be a
+        symmetric sparse MatrixOperator and A(mu) SPD.  It keeps 5 blocks (P, n) and is the cheaper
+        method per iteration.
+        method='gmres': restarted GMRES(m) in the R inner product (fom_solve.affine_gmres), m =
+        `restart` (default 30).  A(mu) may be non-symmetric or indefinite (convection, Helmholtz-type
+        reaction); the minres ROM (SketchedReductor(projection='minres')) is the reduced counterpart.
+        It keeps 2 m + 5 blocks (rows are solved in chunks to bound that) and does about j + 3
+        passes over (P, n) blocks in step j.
+        The choice is the caller's: whether A(mu) is SPD cannot be observed before solving, and
+        symmetric terms include indefinite operators, on which CG breaks down.
+
+        A row that does not converge within `maxiter` iterations or breaks down raises RlaError;
+        with check=False it is returned as is (its last iterate, or NaN after a breakdown)."""
         from . import fom_solve
+        if method not in ('cg', 'gmres'):
+            raise ValueError(f"solve_batch: method={method!r}, expected 'cg' or 'gmres'")
+        if method == 'cg' and restart is not None:
+            raise ValueError("solve_batch: restart= applies to method='gmres' only")
+        if method == 'gmres':
+            restart = fom_solve._check_restart(30 if restart is None else restart, "solve_batch")
         dev = self.rhs[0].device if self.rhs else torch.device("cuda", torch.cuda.current_device())
         th, tf = _theta_rows(self, theta_lhs, theta_rhs, mus, len(self.operators), len(self.rhs), dev)
         n = self.solution_space.dim
@@ -114,8 +132,12 @@ class AffineModel:
             x0 = fom_solve.check_block(x0, th.shape[0], n, "x0", dev)
         if self._affine is None:
             self._affine = fom_solve.AffineCsr(self.operators)               # once per model
-        X = fom_solve.affine_cg(self._affine, self.rhs, th, tf, preconditioner, tol=tol, maxiter=maxiter, x0=x0,
-                                check=check)[0]
+        if method == 'gmres':
+            X = fom_solve.affine_gmres(self._affine, self.rhs, th, tf, preconditioner, tol=tol, restart=restart,
+                                       maxiter=maxiter, x0=x0, check=check)[0]
+        else:
+            X = fom_solve.affine_cg(self._affine, self.rhs, th, tf, preconditioner, tol=tol, maxiter=maxiter, x0=x0,
+                                    check=check)[0]
         return DeviceVectorArray(self.solution_space, X)
 
 
