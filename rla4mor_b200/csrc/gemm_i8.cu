@@ -49,13 +49,17 @@
 //   warps 8..13  producers: the 64 x 32 Theta tile of the stage (Philox + Box-Muller, rng.cuh), its
 //                8 slices written straight into the 32-byte-swizzled K-major layout
 //   warp 14      bulk copy of the 8 U slices of the stage (32 KB, contiguous in the workspace)
-//   warp 15      MMA: one thread issues 36 tcgen05.mma.kind::i8 (M = 128, N = 64, K = 32) per stage
+//   warp 15      MMA: one thread issues the 36 slice products of a stage as 12 tcgen05.mma.kind::i8
+//                (M = 128, K = 32, N = 64 (8 - i) split at 256: U slice i against B slices 0 .. 7 - i)
 // Cluster pairs along m share the Theta tile as in gemm32.cu: each CTA generates 32 of its 64 rows and
 // pushes their slices to the peer (DSMEM bulk copies that signal the peer's full barrier).
-// Measured on one B200 (1000 W limit), C2 shape (2^22 x 512, k = 2000): 160 ms per step, the board at
-// its power cap (sw_power_cap, ~990 W) -- FP64 DMMA: 240 ms.  Dead ends: U slices read with a 3-D TMA
-// box of 32-byte rows, 390 ms (hence the pre-pass writes each stage's 32 KB contiguously); clusters of
-// four CTAs sharing Theta (16 rows each), 174 ms.
+// Measured on one B200 (1000 W limit), C2 shape (2^22 x 512, k = 2000): 146 ms per step (this kernel
+// 126 ms), the board at its power cap (sw_power_cap, ~995 W) -- FP64 DMMA: 240 ms.  The same products
+// as 36 MMAs of N = 64 took 160 ms per step: the MMAs cost per instruction, about 60 cycles for one of
+// 128 x 64 x 32 (tools/micro/i8_probe.cu).  Dead ends: U slices read with a 3-D TMA box of 32-byte
+// rows, 390 ms (hence the pre-pass writes each stage's 32 KB contiguously); clusters of four CTAs
+// sharing Theta (16 rows each), 174 ms; the 36 MMAs with A-collector reuse and the pair as one 2-CTA
+// MMA (M = 256, no DSMEM push), 157 ms.
 #include "common.cuh"
 #include "rng.cuh"
 #include <algorithm>
@@ -111,13 +115,39 @@ __device__ __forceinline__ uint64_t desc_sw32(uint32_t smem_addr) {
     return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | (uint64_t(1) << 16) | (uint64_t(256 >> 4) << 32) |
            (uint64_t(1) << 46) | (uint64_t(6) << 61);
 }
-// D (int32, TMEM) (+)= A (s8, smem) * B (s8, smem)^T
+// D (int32, TMEM) (+)= A (s8, smem) * B (s8, smem)^T.  COLL, the A collector: 0 A read from shared
+// memory; 1 read and kept (fill); 3 the kept A, for the last time (lastuse)
+#define RLA_UMMA_I8(QUAL)                                                                              \
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::i8" QUAL " [%0], %1, %2, %3, p;\n\t}" \
+                 ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory")
+template <int COLL>
 __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+    static_assert(COLL == 0 || COLL == 1 || COLL == 3, "collector mode");
+    if constexpr (COLL == 0) RLA_UMMA_I8("");
+    else if constexpr (COLL == 1) RLA_UMMA_I8(".collector::a::fill");
+    else RLA_UMMA_I8(".collector::a::lastuse");
+}
+#undef RLA_UMMA_I8
+// The 36 slice products of one stage as 12 MMAs.  The products A_i B_j (j = 0 .. IS - 1 - i) go to
+// levels i .. IS - 1, which are consecutive 64-column groups of TMEM, and the B slices B_j are
+// consecutive 64-row groups of one K-major tile; so one MMA with N = 64 (IS - i) does them all, split
+// at the N <= 256 of the instruction (a second part reuses A from the collector).  Every level is first
+// written at i = 0.  The sums per level are exact int32 sums: the order does not change the result.
+template <int I = 0>
+__device__ __forceinline__ void stage_mmas(uint32_t tmem_base, uint32_t a_addr, uint32_t b_addr, bool first) {
+    if constexpr (I < IS) {
+        constexpr int NS = IS - I;                       // B slices this U slice meets
+        constexpr int N0 = NS < 4 ? NS : 4, N1 = NS - N0;    // slices per MMA (N = 64 per slice, <= 256)
+        // kind::i8, int32 accumulate, A and B signed and K-major, M = 128 (cute::UMMA::InstrDescriptor)
+        constexpr uint32_t id_base = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(IBM >> 4) << 24);
+        constexpr uint32_t id0 = id_base | ((uint32_t)(N0 * IBN >> 3) << 17), id1 = id_base | ((uint32_t)(N1 * IBN >> 3) << 17);
+        const uint32_t acc = (first && I == 0) ? 0u : 1u;
+        const uint64_t adesc = desc_sw32(a_addr + I * IA_SLICE);
+        umma_i8<N1 ? 1 : 0>(tmem_base + (uint32_t)(I * IBN), adesc, desc_sw32(b_addr), id0, acc);
+        if constexpr (N1 > 0)
+            umma_i8<3>(tmem_base + (uint32_t)((I + N0) * IBN), adesc, desc_sw32(b_addr + N0 * IB_SLICE), id1, acc);
+        stage_mmas<I + 1>(tmem_base, a_addr, b_addr, first);
+    }
 }
 __device__ __forceinline__ void umma_commit(uint64_t *bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s32(bar)) : "memory");
@@ -396,8 +426,6 @@ sketch_gemm_i8_kernel(const GemmI8Args a) {
         // ------------------------------------------------------------ MMA issue
         asm volatile("setmaxnreg.dec.sync.aligned.u32 80;");
         if (lane == 0) {
-            // kind::i8, int32 accumulate, A and B signed and K-major, M = 128, N = 64 (cute::UMMA::InstrDescriptor)
-            constexpr uint32_t idesc = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(IBN >> 3) << 17) | ((uint32_t)(IBM >> 4) << 24);
             const uint32_t sbase = s32(smem);
             for (int it = 0; it < iters; ++it) {
                 const int s = it % ISTAGES;
@@ -410,13 +438,7 @@ sketch_gemm_i8_kernel(const GemmI8Args a) {
                 mbar_wait(&full[s], (uint32_t)(it / ISTAGES) & 1u);
                 fence_after();
                 const uint32_t st = sbase + (uint32_t)(s * ISTAGE_BYTES);
-#pragma unroll
-                for (int l = 0; l < IS; ++l) {
-#pragma unroll
-                    for (int i = 0; i <= l; ++i)
-                        umma_i8(tmem_base + (uint32_t)(l * IBN), desc_sw32(st + i * IA_SLICE),
-                                desc_sw32(st + IA_BYTES + (l - i) * IB_SLICE), idesc, (first && i == 0) ? 0u : 1u);
-                }
+                stage_mmas(tmem_base, st, st + IA_BYTES, first);
                 if (CL > 1) umma_commit_all(&empty[s], (uint16_t)((1u << CL) - 1)); else umma_commit(&empty[s]);
                 if ((it % ISPB) == ISPB - 1 || it == iters - 1) umma_commit(&tmem_full);
             }
