@@ -13,8 +13,9 @@ from .vectorarray import DeviceVectorSpace, DeviceVectorArray, IdentityOperator,
 from .embeddings import (RandomEmbedding, SrhtEmbedding, GaussianEmbedding, IdentityEmbedding,  # noqa: F401
                          EmbeddingVectorized, BlockGaussianEmbedding, FrozenDict)
 from .sketched_reductor import SketchedReductor  # noqa: F401
+from .greedy import rb_greedy  # noqa: F401
 
 __all__ = ["RandomEmbedding", "SrhtEmbedding", "GaussianEmbedding", "IdentityEmbedding", "EmbeddingVectorized",
-           "BlockGaussianEmbedding", "SketchedReductor", "DeviceVectorSpace", "DeviceVectorArray",
+           "BlockGaussianEmbedding", "SketchedReductor", "rb_greedy", "DeviceVectorSpace", "DeviceVectorArray",
            "IdentityOperator", "MatrixOperator","srht", "fht_oop", "fht_ip", "SrhtPlan", "get_plan", "draw_signs_and_indices",
            "RlaError", "lib"]

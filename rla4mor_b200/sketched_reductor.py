@@ -118,27 +118,33 @@ class AffineModel:
 
         A row that does not converge within `maxiter` iterations or breaks down raises RlaError;
         with check=False it is returned as is (its last iterate, or NaN after a breakdown)."""
-        from . import fom_solve
-        if method not in ('cg', 'gmres'):
-            raise ValueError(f"solve_batch: method={method!r}, expected 'cg' or 'gmres'")
-        if method == 'cg' and restart is not None:
-            raise ValueError("solve_batch: restart= applies to method='gmres' only")
-        if method == 'gmres':
-            restart = fom_solve._check_restart(30 if restart is None else restart, "solve_batch")
-        dev = self.rhs[0].device if self.rhs else torch.device("cuda", torch.cuda.current_device())
-        th, tf = _theta_rows(self, theta_lhs, theta_rhs, mus, len(self.operators), len(self.rhs), dev)
-        n = self.solution_space.dim
-        if x0 is not None:
-            x0 = fom_solve.check_block(x0, th.shape[0], n, "x0", dev)
-        if self._affine is None:
-            self._affine = fom_solve.AffineCsr(self.operators)               # once per model
-        if method == 'gmres':
-            X = fom_solve.affine_gmres(self._affine, self.rhs, th, tf, preconditioner, tol=tol, restart=restart,
-                                       maxiter=maxiter, x0=x0, check=check)[0]
-        else:
-            X = fom_solve.affine_cg(self._affine, self.rhs, th, tf, preconditioner, tol=tol, maxiter=maxiter, x0=x0,
-                                    check=check)[0]
+        X = solve_rows(self, mus, theta_lhs, theta_rhs, preconditioner=preconditioner, tol=tol, maxiter=maxiter,
+                       x0=x0, check=check, method=method, restart=restart)[0]
         return DeviceVectorArray(self.solution_space, X)
+
+
+def solve_rows(fom, mus, theta_lhs, theta_rhs, *, preconditioner, tol, maxiter, x0, check, method, restart):
+    """AffineModel.solve_batch of the model `fom`, with the solver's per-row results:
+    (X (P, n), iters, resid, info) of fom_solve.affine_cg / affine_gmres."""
+    from . import fom_solve
+    if method not in ('cg', 'gmres'):
+        raise ValueError(f"solve_batch: method={method!r}, expected 'cg' or 'gmres'")
+    if method == 'cg' and restart is not None:
+        raise ValueError("solve_batch: restart= applies to method='gmres' only")
+    if method == 'gmres':
+        restart = fom_solve._check_restart(30 if restart is None else restart, "solve_batch")
+    dev = fom.rhs[0].device if fom.rhs else torch.device("cuda", torch.cuda.current_device())
+    th, tf = _theta_rows(fom, theta_lhs, theta_rhs, mus, len(fom.operators), len(fom.rhs), dev)
+    n = fom.solution_space.dim
+    if x0 is not None:
+        x0 = fom_solve.check_block(x0, th.shape[0], n, "x0", dev)
+    if fom._affine is None:
+        fom._affine = fom_solve.AffineCsr(fom.operators)               # once per model
+    if method == 'gmres':
+        return fom_solve.affine_gmres(fom._affine, fom.rhs, th, tf, preconditioner, tol=tol, restart=restart,
+                                      maxiter=maxiter, x0=x0, check=check)
+    return fom_solve.affine_cg(fom._affine, fom.rhs, th, tf, preconditioner, tol=tol, maxiter=maxiter, x0=x0,
+                               check=check)
 
 
 class SketchedReductor:
